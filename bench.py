@@ -21,6 +21,11 @@ The other mode is measured in the same run and reported under ``details.other_sc
 `parity` : gate run with every benchmark on rank 0 (SURVEY 8d): >= 64 genomes of the timed batch against the exact
            integer oracle (oracle.exact_*; test infrastructure used as the checker only), one full-size Gram compared
            bit for bit, and the default path against the fp64 Cholesky path.  A failed gate exits non-zero.
+
+--dump-outputs DIR writes the fitness the last timed step returned, float64: DIR/fitness.npy for `value` and
+DIR/fitness_e2e.npy for `e2e`, (P, folds) each.  With --impl reference, DIR/fitness.npy alone holds the per-individual
+fitness of the timed sample, one column (the reference scores an individual by its mean over the folds).  Data and
+genomes are seeded, so two builds run with the same arguments can be compared file for file.
 """
 import argparse
 import json
@@ -93,7 +98,29 @@ def parse():
     ap.add_argument("--opt", action="append", default=[], help="engine option name=value (A/B experiments), e.g. fuse_in_gram=1")
     ap.add_argument("--cpu-kind", default="auto", choices=["auto", "reference", "port"],
                     help="CPU arm: the staged reference's own evaluator + worker pool (oracle/_ref), or the oracle port")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the fitness the timed path returned in its last step as DIR/<name>.npy (float64)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
+
+
+DUMP_BUDGET_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, arrays):
+    """Save each array as out_dir/<name>.npy in float64.  The arrays share a 64 MB budget: an array over its share keeps
+    a fixed, seeded sample of its rows, so two builds run with the same arguments dump the same rows."""
+    os.makedirs(out_dir, exist_ok=True)
+    share = DUMP_BUDGET_BYTES // max(1, len(arrays))
+    for name, a in arrays.items():
+        a = np.asarray(a, dtype=np.float64)
+        if a.nbytes > share:
+            row_bytes = max(1, a.nbytes // a.shape[0])
+            rows = np.random.default_rng(0).choice(a.shape[0], size=share // row_bytes, replace=False)
+            a = a[np.sort(rows)]
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 # ------------------------------------------------------------------------------------------------
@@ -385,11 +412,13 @@ def reference_main(args, wl, rank, cores):
             pos += sample
         t = 0.0
         for _ in range(args.steps):
-            dt, _f = arm.step(gens[pos:pos + sample])
+            dt, fit = arm.step(gens[pos:pos + sample])
             t += dt
             pos += sample
     finally:
         arm.close()
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"fitness": np.asarray(fit, dtype=np.float64).reshape(-1, 1)})
     value = sample * folds * args.steps / t
     line = {
         "impl": "reference", "metric": METRIC, "value": value, "unit": UNIT, "n_gpus": args.gpus,
@@ -517,11 +546,16 @@ def main():
         barrier()
         clocks = sampler.result()
         ms = e0.elapsed_time(e1)
+        fit_resident = None
+        if args.dump_outputs:
+            # (p_total, S) as the last timed step left it; the instrumented pass below overwrites the buffer
+            got = (fit_all if world > 1 else fit_dev).cpu().numpy().reshape(world, widest, S)
+            fit_resident = np.concatenate([got[r, :cuts[r + 1] - cuts[r]] for r in range(world)])
         launches = eng.launch_count()
         facts = {q: bool(eng.info(q)) for q in ("last_c16", "last_fused_scale", "last_fp4")}   # of the TIMED pass
         wave, precision = eng.last_wave(), eng.last_precision()
         res = {"p_total": p_total, "p_local": hi - lo, "launches": launches, "clocks": clocks, "facts": facts,
-               "wave": wave, "precision": precision, "pinned": pinned, "cuts": cuts}
+               "wave": wave, "precision": precision, "pinned": pinned, "cuts": cuts, "fit_last_resident": fit_resident}
         if profile:
             eng.set_option("profile", 1)
             eng.reset_counters()
@@ -807,6 +841,8 @@ def main():
             "parity": parity,
             "parity_ok": parity_ok if (parity is not None or cpu_baseline is not None) else None,
         }
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, {"fitness": prim["fit_last_resident"], "fitness_e2e": prim["fit_last_e2e"]})
         print(json.dumps(line))
     eng.close()
     if world > 1:

@@ -3,8 +3,8 @@
 data set and seed -- once with the reference's own CPU evaluator (its worker pool), once with the B200 evaluators
 plugged in through ``python -m tblup_b200.main`` -- and the two result directories compared generation by generation:
 ``<seed>_results.csv`` (values rounded to 4 decimals by the reference's monitor) and the selected panels in
-``<seed>_archive.json``.  The reference is imported from the live checkout (build container) or from the mirror that
-``oracle/stage_ref.py`` stages under ``oracle/_ref`` (GPU box).
+``<seed>_archive.json``.  The reference is imported from a checkout (``TBLUP_REFERENCE``, else BASELINE.json's
+``reference_path``) or from the mirror that ``oracle/stage_ref.py`` stages under ``oracle/_ref``.
 
     python scripts/main_c1.py                      # 1 000 x 10 000, --features 1500 --population_size 50 --generations 10
     python scripts/main_c1.py --regressor intracv_blup --cv_folds 5 --generations 4
@@ -37,7 +37,8 @@ def run_pair(n=1000, m=10000, features=1500, pop=50, gens=10, seed=0, extra=(), 
     from tblup_b200 import synth
     ref = stage_ref.ref_path()
     if ref is None:
-        raise RuntimeError("reference not available (neither /root/reference nor oracle/_ref)")
+        raise RuntimeError("reference not available (no checkout at TBLUP_REFERENCE or BASELINE.json's "
+                           "reference_path, no mirror under oracle/_ref)")
     own_tmp = None
     if workdir is None:
         own_tmp = tempfile.TemporaryDirectory()

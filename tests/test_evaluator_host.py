@@ -11,9 +11,10 @@ import pytest
 
 from conftest import load_golden, unpack
 from fake_engine import OracleEngine
+from oracle import stage_ref
 
-REF = os.environ.get("TBLUP_REFERENCE", "/root/reference")
-HAVE_REF = os.path.isdir(os.path.join(REF, "tblup"))
+REF = stage_ref.ref_path()
+HAVE_REF = REF is not None
 
 
 class Indv:
@@ -288,7 +289,7 @@ def test_evaluator_shards_over_torch_distributed_ranks_gloo(tmp_path):
     assert np.abs(np.array([p.fitness for p in pop]) - np.array(got[0][0])).max() < 1e-12
 
 
-@pytest.mark.skipif(not HAVE_REF, reason="reference checkout not present (GPU box)")
+@pytest.mark.skipif(not HAVE_REF, reason="no reference checkout or oracle/_ref mirror (oracle/stage_ref.py)")
 @pytest.mark.parametrize("name", ["traj_gblup", "traj_intracv"])
 def test_reference_main_loop_drives_our_evaluator(name, tmp_path, monkeypatch):
     """The UNMODIFIED reference Population / evolver / selector / monitor, wired by its own build_kwargs, with our

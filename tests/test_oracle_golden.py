@@ -4,13 +4,12 @@ Both layers are pinned: the reference-faithful restatement must reproduce the re
 rounding noise, and the exact-integer restatement (the specification of the CUDA kernels) must agree
 with them far inside the 1e-6 fitness tolerance of BASELINE.json's north_star.
 """
-import os
-
 import numpy as np
 import pytest
 
 from conftest import load_golden, unpack
 from oracle import gblup_oracle as O
+from oracle import stage_ref
 
 FIT_CASES = ["fit_small", "fit_offset", "fit_mid"]
 
@@ -87,15 +86,17 @@ def test_pearson_conventions():
     assert np.isnan(O.pearson_abs(np.ones(5), np.arange(5.0)))
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/tblup"), reason="reference checkout not present")
+@pytest.mark.skipif(stage_ref.ref_path() is None,
+                    reason="no reference checkout or oracle/_ref mirror (oracle/stage_ref.py)")
 def test_removal_restatement_matches_reference_handler():
     """oracle/de_oracle.py's SNP-removal helpers against the live tblup.evaluator.SNPRemovalHandler."""
     import sys
-    sys.path.insert(0, "/root/reference")
+    ref = stage_ref.ref_path()
+    sys.path.insert(0, ref)
     try:
         from tblup.evaluator import SNPRemovalHandler
     finally:
-        sys.path.remove("/root/reference")
+        sys.path.remove(ref)
     from oracle import de_oracle as D
 
     class Indv:
