@@ -135,6 +135,9 @@ int tb_debug_fetch(tb_ctx* ctx, int what, int job, void* out, size_t nbytes);
  * "solve_pair" (0 = one CTA per matrix, 2 = a cluster of two, 1 = by batch size [default]),
  * "t16" (0/1, default 1: the entries of a Cholesky block column below its diagonal block are kept as halves between
  * the update that forms them and the panel GEMM that finishes them in place; 0 = fp32 / TF32 as in the first version),
+ * "panel_fused" (0/1, default 1: with t16, those entries are formed and finished in ONE launch after the diagonal
+ * chain -- update, then product with the inverse of the diagonal block, the intermediate kept in shared memory; the
+ * factor is bit-identical to 0 = the update of the whole block column, then the panel GEMM as its own launch),
  * "epi_warps" (8 or 16 [default]: epilogue warps of the Cholesky GEMM kernel), "chain_fused" (the 64 x 64
  * diagonal-block chain of a block column runs as ONE shared-memory kernel for waves of at most this many jobs;
  * -1 = the SM count [default], 0 = never), "chain_inverse" (0/1, default 1: that kernel also forms the inverse of the
@@ -142,7 +145,7 @@ int tb_debug_fetch(tb_ctx* ctx, int what, int job, void* out, size_t nbytes);
 int tb_set_option(tb_ctx* ctx, const char* name, long long value);
 
 /* Facts about the last evaluation / the context: "last_c16", "last_fused_scale", "last_mixed", "last_wave",
- * "storage", "wide_panel", "de_removed" (size of the removed-marker set), "staged" (genomes staged), "last_fp4", "last_perm", "last_split",
+ * "storage", "wide_panel", "panel_fused", "de_removed" (size of the removed-marker set), "staged" (genomes staged), "last_fp4", "last_perm", "last_split",
  * "last_fallbacks" (jobs of the last evaluation whose mixed-precision solve gave up -- pivot breakdown or no
  * convergence, h2 close to 1 -- and that were evaluated again with the fp64 Cholesky). */
 int tb_get_info(const tb_ctx* ctx, const char* name, long long* value);

@@ -533,7 +533,8 @@ int eval_core(TbCtx* c, const int32_t* slots, int n_slots, double h2, int mode_r
         MarkCtx mc{c, 0};
         cudaError_t ce = tb_chol_tc_factor(d_L32, d_Linv32, d_L16, d_Linv256, d_status, n_jobs, max_ntp, c->n_sm, st, nl, &e,
                                            c->profile ? &mark_cb : nullptr, &mc, from_c ? &fc : nullptr, c->t16, c->epi_warps,
-                                           (c->chain_fused < 0 ? c->n_sm : c->chain_fused) * (c->chain_inverse ? 1 : -1));
+                                           (c->chain_fused < 0 ? c->n_sm : c->chain_fused) * (c->chain_inverse ? 1 : -1),
+                                           c->panel_fused);
         if (ce != cudaSuccess)
           return fail(c, "tensor-core Cholesky: " + (e.empty() ? std::string(cudaGetErrorString(ce)) : e), -2);
         count(c, TB_ST_CHOL_UPDATE, mc.n_update);
@@ -1377,6 +1378,7 @@ int tb_set_option(tb_ctx* c, const char* name, long long value) {
   else if (s == "chain_inverse") c->chain_inverse = value != 0;  // A/B: 0 = trinv256_kernel after the fused chain
   else if (s == "chain_fused") c->chain_fused = (int)value;      // jobs per wave up to which the diagonal-block chain is one launch (-1: SM count, 0: never)
   else if (s == "t16") c->t16 = value != 0;                     // A/B: 0 = fp32 block columns all the way down (round-2 first version)
+  else if (s == "panel_fused") c->panel_fused = value != 0;     // A/B: 0 = update, then the wide panel GEMM as its own launch
   else if (s == "narrow_c") c->narrow_c = value != 0;
   else if (s == "gram_fp4") c->gram_fp4 = value != 0;
   else if (s == "perm_rows") c->perm_rows = value != 0;
@@ -1395,6 +1397,7 @@ int tb_get_info(const tb_ctx* c, const char* name, long long* value) {
   else if (s == "storage") *value = c->storage;
   else if (s == "wide_panel") *value = c->wide_panel;
   else if (s == "t16") *value = c->t16;
+  else if (s == "panel_fused") *value = c->panel_fused;
   else if (s == "epi_warps") *value = c->epi_warps;
   else if (s == "de_removed") *value = c->de.n_banned;
   else if (s == "last_fp4") *value = c->last_fp4;

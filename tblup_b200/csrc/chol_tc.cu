@@ -113,6 +113,13 @@ __device__ __forceinline__ float round_tf32(float x) {
   return __uint_as_float(r);
 }
 
+// A cross-product as a float.  Integers below 2^23: 0x4b000000 | c is the float 2^23 + c (no converter pipe); one byte
+// permute per int16 half of a word.
+__device__ __forceinline__ float c_from_i16(uint32_t w, bool hi) {
+  return __uint_as_float(__byte_perm(w, 0x4b000000u, hi ? 0x7432 : 0x7410)) - 8388608.f;
+}
+__device__ __forceinline__ float c_from_i32(uint32_t w) { return __uint_as_float(0x4b000000u | w) - 8388608.f; }
+
 // SRC: where update mode reads the entries it modifies -- 0: the fp32 matrix L32, 1: int16 cross-products, 2: int32
 // cross-products (TbFromC: the scaled matrix is formed on the fly)
 template <bool F16, int SRC, int EW>
@@ -316,17 +323,16 @@ tf32_gemm_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_consta
               const float4 raw = cv[i][j >> 1];
               const uint32_t w0 = (j & 1) ? __float_as_uint(raw.z) : __float_as_uint(raw.x);
               const uint32_t w1 = (j & 1) ? __float_as_uint(raw.w) : __float_as_uint(raw.y);
-              // integers below 2^23: 0x4b000000 | c is the float 2^23 + c (no converter pipe); one byte permute each
-              cx[0] = __uint_as_float(__byte_perm(w0, 0x4b000000u, 0x7410)) - 8388608.f;
-              cx[1] = __uint_as_float(__byte_perm(w0, 0x4b000000u, 0x7432)) - 8388608.f;
-              cx[2] = __uint_as_float(__byte_perm(w1, 0x4b000000u, 0x7410)) - 8388608.f;
-              cx[3] = __uint_as_float(__byte_perm(w1, 0x4b000000u, 0x7432)) - 8388608.f;
+              cx[0] = c_from_i16(w0, false);
+              cx[1] = c_from_i16(w0, true);
+              cx[2] = c_from_i16(w1, false);
+              cx[3] = c_from_i16(w1, true);
             } else {
               const float4 raw = cv[i][SRC == 1 ? 0 : j];
-              cx[0] = __uint_as_float(0x4b000000u | __float_as_uint(raw.x)) - 8388608.f;
-              cx[1] = __uint_as_float(0x4b000000u | __float_as_uint(raw.y)) - 8388608.f;
-              cx[2] = __uint_as_float(0x4b000000u | __float_as_uint(raw.z)) - 8388608.f;
-              cx[3] = __uint_as_float(0x4b000000u | __float_as_uint(raw.w)) - 8388608.f;
+              cx[0] = c_from_i32(__float_as_uint(raw.x));
+              cx[1] = c_from_i32(__float_as_uint(raw.y));
+              cx[2] = c_from_i32(__float_as_uint(raw.z));
+              cx[3] = c_from_i32(__float_as_uint(raw.w));
             }
             const float ctv[4] = {ct.x, ct.y, ct.z, ct.w};
             if (pad_warp) {
@@ -402,6 +408,331 @@ tf32_gemm_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_consta
         acc_phase ^= 1;
       }
     }
+  }
+
+  tc_fence_before();
+  __syncthreads();
+  if (warp == 1) {
+    tc_fence_after();
+    tmem_dealloc<TACC * MAX_N>(tmem_base);
+  }
+}
+
+// The rows below the 256-row diagonal block of a wide block column formed from the cross-products, finished in ONE
+// launch (option panel_fused).  Per 128 x 256 tile:
+//   phase 1  T = A - L[:, 0:c0] L[J, 0:c0]^T   the outer update and its epilogue; T, rounded to halves, goes into a
+//                                              shared-memory tile laid out as the K-major SWIZZLE_128B MMA operand
+//   phase 2  L = T X^T                         X = the fp16 inverse of the diagonal block (K = 256); the rounded factor
+//                                              entries go back into the same buffer and leave by TMA store into L16
+// Same operands, MMA shapes and K order as the update (t16) + wide panel GEMM (f16ops) pair, so the factor is
+// bit-identical; T no longer makes a round trip through L16 (2 + 2 bytes per entry) and the panel launch is gone.
+// Shared memory: a 3-stage ring (144 KB; phase 2 only fills the B slots) + the 64 KB T tile.  Both TMEM accumulators
+// are used: phase 2 of tile k reuses tile k's accumulator once phase 1's epilogue has drained it, and the MMA warp
+// issues phase 1 of tile k + 1 BEFORE phase 2 of tile k, so the tensor pipe runs the long product while the epilogue
+// stages T (the epilogue, which reads the cross-products, is the longer of the two).
+constexpr int FSTAGES = 3;
+constexpr int FT_KB_BYTES = TBM * 128;              // one 64-half k-block of the T tile
+constexpr int FT_BYTES = 4 * FT_KB_BYTES;           // 64 KiB
+constexpr int F_SMEM = FSTAGES * TSTAGE_BYTES + FT_BYTES + 1024 + 256;
+
+struct FBarriers {
+  uint64_t full[FSTAGES];
+  uint64_t empty[FSTAGES];
+  uint64_t p1_full[TACC];      // phase 1 product of the tile in accumulator a complete
+  uint64_t p2_full[TACC];      // phase 2 product complete (the T tile has been read)
+  uint64_t acc_empty[TACC];
+  uint64_t t_full;             // the T tile is in shared memory
+  uint32_t tmem_base;
+};
+static_assert(sizeof(FBarriers) <= 256, "barrier block");
+
+template <int SRC, int EW>
+__global__ void __launch_bounds__(t_threads(EW), 1)
+panel_fused_kernel(const __grid_constant__ CUtensorMap tmap_l, const __grid_constant__ CUtensorMap tmap_x,
+                   const __grid_constant__ GemmParams p) {
+  extern __shared__ uint8_t smem_raw[];
+  uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
+  uint8_t* tbuf = smem + FSTAGES * TSTAGE_BYTES;
+  FBarriers* bars = reinterpret_cast<FBarriers*>(tbuf + FT_BYTES);
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  const int n_items = p.n_jobs * p.n_mtiles;
+  const int nkb1 = p.K / HBK;                       // phase 1 k-blocks (0 for block column 0: T is A itself)
+  constexpr int NKB2 = 256 / HBK;
+  const int n_my = blockIdx.x < n_items ? (n_items - blockIdx.x + gridDim.x - 1) / gridDim.x : 0;
+
+  if (warp == 0 && lane == 0) {
+    prefetch_tensormap(&tmap_l);
+    prefetch_tensormap(&tmap_x);
+    for (int s = 0; s < FSTAGES; ++s) {
+      mbar_init(&bars->full[s], 1);
+      mbar_init(&bars->empty[s], 1);
+    }
+    for (int s = 0; s < TACC; ++s) {
+      mbar_init(&bars->p1_full[s], 1);
+      mbar_init(&bars->p2_full[s], 1);
+      mbar_init(&bars->acc_empty[s], EW);
+    }
+    mbar_init(&bars->t_full, EW);
+    fence_barrier_init();
+  }
+  if (warp == 1) tmem_alloc<TACC * MAX_N>(&bars->tmem_base);
+  tc_fence_before();
+  __syncthreads();
+  tc_fence_after();
+  const uint32_t tmem_base = bars->tmem_base;
+
+  // ring order, shared by the producer and the MMA issuer: P1(0), then P1(k + 1), P2(k) for k = 0, 1, ...
+  if (warp == 0) {
+    if (lane == 0) {
+      int stage = 0;
+      uint32_t phase = 0;
+      auto next = [&]() {
+        if (++stage == FSTAGES) {
+          stage = 0;
+          phase ^= 1;
+        }
+      };
+      auto load_p1 = [&](int k) {
+        const int item = blockIdx.x + k * gridDim.x;
+        const int job = item / p.n_mtiles, mt = item - job * p.n_mtiles;
+        const int row_a = job * p.ntp + p.row0 + mt * TBM, row_b = job * p.ntp + p.c_col0;
+        for (int kb = 0; kb < nkb1; ++kb) {
+          mbar_wait(&bars->empty[stage], phase ^ 1);
+          uint8_t* sa = smem + stage * TSTAGE_BYTES;
+          mbar_arrive_expect_tx(&bars->full[stage], TA_BYTES + 4 * BOX_BYTES);
+          tma_load_2d(sa, &tmap_l, &bars->full[stage], kb * HBK, row_a);
+          tma_load_2d(sa + BOX_BYTES, &tmap_l, &bars->full[stage], kb * HBK, row_a + BOX_ROWS);
+          for (int b = 0; b < 4; ++b)
+            tma_load_2d(sa + TA_BYTES + b * BOX_BYTES, &tmap_l, &bars->full[stage], kb * HBK, row_b + b * BOX_ROWS);
+          next();
+        }
+      };
+      auto load_p2 = [&](int k) {
+        const int job = (blockIdx.x + k * gridDim.x) / p.n_mtiles;
+        for (int kb = 0; kb < NKB2; ++kb) {
+          mbar_wait(&bars->empty[stage], phase ^ 1);
+          uint8_t* sb = smem + stage * TSTAGE_BYTES + TA_BYTES;
+          mbar_arrive_expect_tx(&bars->full[stage], 4 * BOX_BYTES);
+          for (int b = 0; b < 4; ++b)
+            tma_load_2d(sb + b * BOX_BYTES, &tmap_x, &bars->full[stage], kb * HBK, job * 256 + b * BOX_ROWS);
+          next();
+        }
+      };
+      if (n_my > 0) load_p1(0);
+      for (int k = 0; k < n_my; ++k) {
+        if (k + 1 < n_my) load_p1(k + 1);
+        load_p2(k);
+      }
+    }
+  } else if (warp == 1) {
+    if (lane == 0) {
+      const uint32_t idesc = umma_idesc_f16(TBM, 256);
+      int stage = 0;
+      uint32_t phase = 0;
+      auto kblock = [&](uint32_t tmem_d, uint32_t sa, int kb) {
+        mbar_wait(&bars->full[stage], phase);
+        tc_fence_after();
+        const uint64_t adesc = umma_desc_k_sw128(sa);
+        const uint64_t bdesc = umma_desc_k_sw128(smem_u32(smem + stage * TSTAGE_BYTES + TA_BYTES));
+#pragma unroll
+        for (int k = 0; k < 4; ++k) umma_f16(tmem_d, adesc + 2 * k, bdesc + 2 * k, idesc, (kb | k) != 0);
+        umma_commit(&bars->empty[stage]);
+        if (++stage == FSTAGES) {
+          stage = 0;
+          phase ^= 1;
+        }
+      };
+      auto claim = [&](int k) {                     // first use of tile k's accumulator
+        mbar_wait(&bars->acc_empty[k & 1], ((k >> 1) & 1) ^ 1);
+        tc_fence_after();
+      };
+      auto p1 = [&](int k) {
+        claim(k);
+        const uint32_t tmem_d = tmem_base + (k & 1) * MAX_N;
+        for (int kb = 0; kb < nkb1; ++kb) kblock(tmem_d, smem_u32(smem + stage * TSTAGE_BYTES), kb);
+        umma_commit(&bars->p1_full[k & 1]);
+      };
+      if (n_my > 0 && nkb1 > 0) p1(0);
+      for (int k = 0; k < n_my; ++k) {
+        if (k + 1 < n_my && nkb1 > 0) p1(k + 1);
+        if (nkb1 == 0) claim(k);
+        mbar_wait(&bars->t_full, k & 1);
+        tc_fence_after();
+        const uint32_t tmem_d = tmem_base + (k & 1) * MAX_N;
+        for (int kb = 0; kb < NKB2; ++kb) kblock(tmem_d, smem_u32(tbuf + kb * FT_KB_BYTES), kb);
+        umma_commit(&bars->p2_full[k & 1]);
+      }
+    }
+  } else {
+    // Epilogue: thread = one row of the tile (TMEM lane quarter q = warp & 3), the EW / 4 warps of a quarter take its
+    // 32-column chunks round-robin as in tf32_gemm_kernel, in units of 16 columns.  The cross-products of PF units are
+    // in flight ahead of their use -- the first ones of the NEXT tile while phase 2 of this one runs -- as many as the
+    // register budget allows without spilling (96 registers per thread at EW = 16, 168 at EW = 8).
+    constexpr int CG = EW / 4;
+    constexpr int NU = 2 * (8 / CG);                              // 16-column units per thread and tile
+    constexpr int CVU = SRC == 1 ? 2 : 4;                         // 16-byte loads per unit
+    constexpr int PF = SRC == 1 ? NU : 2;                         // int16: the whole tile; int32: two units
+    const int q = warp & 3, g = (warp - 2) >> 2;
+    const int tr = q * 32 + lane;                                 // tile row of this thread
+    const uint32_t tsm = smem_u32(tbuf) + tr * 128;
+    const bool storer = warp == 2 && lane == 0;
+    const bool has_acc = nkb1 > 0;
+    uint4 cv[NU][CVU];
+    size_t rowoff = 0;                                            // cross-product row of the tile whose units load next
+    int l_h0 = 0, l_gap = 0, l_nt = 0;
+    // (rows past the job's end are padding rows, r >= n_t: they read panel row 0, so every load is in bounds and
+    // needs no branch)
+    auto tile_src = [&](int item) {
+      const int job = item / p.n_mtiles, mt = item - job * p.n_mtiles;
+      const int r = p.row0 + mt * TBM + tr;
+      const TbFuseCoef cf = p.fc.coef[job];
+      const int rr = r < cf.n_t ? r + (r >= cf.hole0 ? cf.gap : 0) : 0;
+      rowoff = ((size_t)cf.cw * p.fc.rpad + rr) * p.fc.rpad;
+      l_h0 = cf.hole0;
+      l_gap = cf.gap;
+      l_nt = cf.n_t;
+    };
+    auto load_unit = [&](uint4 (&dst)[CVU], int u) {
+      const int b = p.c_col0 + (g + CG * (u >> 1)) * 32 + 16 * (u & 1);
+#pragma unroll
+      for (int j = 0; j < CVU; ++j) {
+        const int bj = b + (SRC == 1 ? 8 : 4) * j;              // (8-column groups never straddle the hole)
+        const int ub = bj + ((bj >= l_h0 && bj < l_nt) ? l_gap : 0);
+        dst[j] = SRC == 1 ? *reinterpret_cast<const uint4*>(static_cast<const int16_t*>(p.fc.C) + rowoff + ub)
+                          : *reinterpret_cast<const uint4*>(static_cast<const int32_t*>(p.fc.C) + rowoff + ub);
+      }
+    };
+    // 16 halves of this thread's row (tile columns col .. col + 15) into the T tile, swizzled as a TMA load would place them
+    auto put_t = [&](int col, const uint32_t (&h)[8]) {
+      const uint32_t base = tsm + (col >> 6) * FT_KB_BYTES;
+      const int c16 = (col & 63) >> 3;
+#pragma unroll
+      for (int s = 0; s < 2; ++s)
+        asm volatile("st.shared.v4.b32 [%0], {%1, %2, %3, %4};" ::"r"(base + (((c16 + s) ^ (tr & 7)) << 4)),
+                     "r"(h[4 * s]), "r"(h[4 * s + 1]), "r"(h[4 * s + 2]), "r"(h[4 * s + 3])
+                     : "memory");
+    };
+    auto epi_sync = [&]() { asm volatile("bar.sync 1, %0;" ::"n"(EW * 32) : "memory"); };
+
+    if (n_my > 0) {
+      tile_src(blockIdx.x);
+#pragma unroll
+      for (int u = 0; u < PF; ++u) load_unit(cv[u], u);
+    }
+    for (int k = 0; k < n_my; ++k) {
+      const int item = blockIdx.x + k * gridDim.x;
+      const int job = item / p.n_mtiles, mt = item - job * p.n_mtiles;
+      const int a = k & 1;
+      const uint32_t par = (k >> 1) & 1;
+      const int r = p.row0 + mt * TBM + tr;
+      const int rw0 = p.row0 + mt * TBM + q * 32;
+      const TbFuseCoef cf = p.fc.coef[job];
+      const float f_scale = cf.scale;
+      const float f_rt = p.fc.terms[(size_t)job * 2 * p.ntp + (r < p.row_end ? r : 0)];
+      const float* f_ct = p.fc.terms + (size_t)job * 2 * p.ntp + p.ntp + p.c_col0;
+      const bool pad_warp = rw0 + 32 > cf.n_t;                   // (warp-uniform) some rows of this warp are padding
+      const bool real_row = r < cf.n_t;
+      const uint32_t tacc = tmem_base + (static_cast<uint32_t>(q * 32) << 16) + a * MAX_N;
+      if (has_acc) {
+        mbar_wait(&bars->p1_full[a], par);
+        tc_fence_after();
+      }
+      if (storer) bulk_wait_group_read0();                        // the previous tile's store has read the buffer
+      epi_sync();
+      // phase 1 epilogue: T = A - acc (every entry lies below the diagonal: no lambda; padding rows are zero)
+#pragma unroll
+      for (int u = 0; u < NU; ++u) {
+        if (u + PF < NU) load_unit(cv[u + PF], u + PF);
+        const int col = (g + CG * (u >> 1)) * 32 + 16 * (u & 1);   // tile column
+        uint32_t v[16];
+        if (has_acc) {
+          tmem_ld_32x16(tacc + col, v);
+          tmem_ld_wait();
+        } else {
+#pragma unroll
+          for (int j = 0; j < 16; ++j) v[j] = 0u;
+        }
+        float o[16];
+#pragma unroll
+        for (int j = 0; j < 4; ++j) {
+          const float4 ct = *reinterpret_cast<const float4*>(f_ct + col + 4 * j);
+          const float ctv[4] = {ct.x, ct.y, ct.z, ct.w};
+          float cx[4];
+          if (SRC == 1) {
+            const uint4 raw = cv[u][j >> 1];
+            const uint32_t w0 = (j & 1) ? raw.z : raw.x, w1 = (j & 1) ? raw.w : raw.y;
+            cx[0] = c_from_i16(w0, false);
+            cx[1] = c_from_i16(w0, true);
+            cx[2] = c_from_i16(w1, false);
+            cx[3] = c_from_i16(w1, true);
+          } else {
+            const uint4 raw = cv[u][SRC == 1 ? 0 : j];
+            cx[0] = c_from_i32(raw.x);
+            cx[1] = c_from_i32(raw.y);
+            cx[2] = c_from_i32(raw.z);
+            cx[3] = c_from_i32(raw.w);
+          }
+#pragma unroll
+          for (int e = 0; e < 4; ++e) {
+            const float av = (!pad_warp || real_row) ? fmaf(cx[e], f_scale, f_rt + ctv[e]) : 0.f;
+            o[4 * j + e] = av - __uint_as_float(v[4 * j + e]);
+          }
+        }
+        uint32_t h[8];
+#pragma unroll
+        for (int j = 0; j < 8; ++j) {
+          const __half2 hh = __floats2half2_rn(o[2 * j], o[2 * j + 1]);
+          h[j] = *reinterpret_cast<const uint32_t*>(&hh);
+        }
+        put_t(col, h);
+      }
+      tc_fence_before();
+      fence_proxy_async_smem();                                   // T is read by the MMA (async proxy)
+      __syncwarp();
+      if (lane == 0) mbar_arrive(&bars->t_full);
+      // the next tile's first cross-products travel while phase 2 runs
+      if (k + 1 < n_my) {
+        tile_src(item + gridDim.x);
+#pragma unroll
+        for (int u = 0; u < PF; ++u) load_unit(cv[u], u);
+      }
+      mbar_wait(&bars->p2_full[a], par);
+      tc_fence_after();
+      // phase 2 epilogue: the final factor entries, rounded as the panel GEMM rounds them (TF32, then half)
+#pragma unroll
+      for (int u = 0; u < NU; ++u) {
+        const int col = (g + CG * (u >> 1)) * 32 + 16 * (u & 1);
+        uint32_t v[16];
+        tmem_ld_32x16(tacc + col, v);
+        tmem_ld_wait();
+        uint32_t h[8];
+#pragma unroll
+        for (int j = 0; j < 8; ++j) {
+          const __half2 hh = __floats2half2_rn(round_tf32(__uint_as_float(v[2 * j])), round_tf32(__uint_as_float(v[2 * j + 1])));
+          h[j] = *reinterpret_cast<const uint32_t*>(&hh);
+        }
+        put_t(col, h);
+      }
+      tc_fence_before();
+      fence_proxy_async_smem();                                   // the tile is read by the TMA store (async proxy)
+      __syncwarp();
+      if (lane == 0) mbar_arrive(&bars->acc_empty[a]);
+      epi_sync();
+      if (storer) {
+        // ntp is a multiple of 64: a 64-row box lies wholly inside or wholly outside the job's rows
+        const int row_t = p.row0 + mt * TBM;
+#pragma unroll
+        for (int hb = 0; hb < 2; ++hb) {
+          if (row_t + hb * BOX_ROWS >= p.row_end) continue;
+#pragma unroll
+          for (int kb = 0; kb < 4; ++kb)
+            tma_store_2d(&tmap_l, tbuf + kb * FT_KB_BYTES + hb * BOX_BYTES, p.c_col0 + kb * HBK,
+                         job * p.ntp + row_t + hb * BOX_ROWS);
+        }
+        bulk_commit_group();
+      }
+    }
+    if (storer) bulk_wait_group0();
   }
 
   tc_fence_before();
@@ -1107,6 +1438,11 @@ cudaError_t tb_chol_tc_init() {
   TB_GEMM_ATTR(false, 0, 8) TB_GEMM_ATTR(true, 0, 8) TB_GEMM_ATTR(true, 1, 8) TB_GEMM_ATTR(true, 2, 8)
   TB_GEMM_ATTR(false, 0, 16) TB_GEMM_ATTR(true, 0, 16) TB_GEMM_ATTR(true, 1, 16) TB_GEMM_ATTR(true, 2, 16)
 #undef TB_GEMM_ATTR
+#define TB_FUSED_ATTR(S, W)                                                                                   \
+  e = cudaFuncSetAttribute(panel_fused_kernel<S, W>, cudaFuncAttributeMaxDynamicSharedMemorySize, F_SMEM); \
+  if (e != cudaSuccess) return e;
+  TB_FUSED_ATTR(1, 8) TB_FUSED_ATTR(2, 8) TB_FUSED_ATTR(1, 16)
+#undef TB_FUSED_ATTR
   return cudaSuccess;
 }
 
@@ -1116,7 +1452,7 @@ cudaError_t tb_chol_tc_init() {
 cudaError_t tb_chol_tc_factor(float* L32, float* Linv32, void* L16, float* Linv256, int* status, int n_jobs, int ntp,
                               int n_sm, cudaStream_t st, int* launches, std::string* err,
                               void (*mark)(void*, int, int), void* mark_ctx, const TbFromC* from_c, int t16, int epi_warps,
-                              int chain_fused_jobs) {
+                              int chain_fused_jobs, int panel_fused) {
   const bool chain_inverse = chain_fused_jobs >= 0;      // (negative: fused chain for -n jobs without the inverse; A/B)
   if (chain_fused_jobs < 0) chain_fused_jobs = -chain_fused_jobs;
   CUtensorMap tm_l, tm_inv, tm_inv256;
@@ -1181,12 +1517,16 @@ cudaError_t tb_chol_tc_factor(float* L32, float* Linv32, void* L16, float* Linv2
     // in fp32: the update writes them as halves into L16, the panel GEMM (fp16 operands) replaces them in place by the
     // factor entries -- 2 + 2 bytes per entry instead of 4 + 4
     const bool col16 = wide && t16 && upd16 && from_c && !(c0 == 0 && from_c->skip_blk0);
+    // ... and those rows can be finished by one launch after the diagonal chain (panel_fused_kernel): the update before
+    // the chain then only covers the diagonal block
+    const bool fused = col16 && panel_fused;
     if (c0 > 0 || (from_c && upd16 && !from_c->skip_blk0)) {
       // (block column 0 with from_c: K = 0, the launch only forms the block column from the cross-products)
       if (mark) mark(mark_ctx, 0, 0);
       GemmParams p{};
       p.row0 = c0; p.a_col0 = 0; p.K = c0; p.b_row0 = c0; p.b_col0 = 0; p.b_rows_per_job = ntp; p.c_col0 = c0;
       p.N = w; p.mode = 0;
+      if (fused) p.row_end = c0 + w;
       if (from_c && upd16) {                       // this launch is the first touch of block column c0: form it from C
         p.from_c = 1;
         p.fc = *from_c;
@@ -1240,13 +1580,13 @@ cudaError_t tb_chol_tc_factor(float* L32, float* Linv32, void* L16, float* Linv2
         if ((e = gemm(tm_inv, p)) != cudaSuccess) return e;
       }
     }
-    if (wide) {
-      if (!chain_has_inverse) {
-        trinv256_kernel<<<n_jobs, 256, TRINV_SMEM, st>>>(L32, Linv32, Linv256,
-                                                         col16 ? reinterpret_cast<__half*>(Linv256) : nullptr, ntp, c0);
-        launches[1]++;
-        if ((e = cudaGetLastError()) != cudaSuccess) return e;
-      }
+    if (wide && !chain_has_inverse) {
+      trinv256_kernel<<<n_jobs, 256, TRINV_SMEM, st>>>(L32, Linv32, Linv256,
+                                                       col16 ? reinterpret_cast<__half*>(Linv256) : nullptr, ntp, c0);
+      launches[1]++;
+      if ((e = cudaGetLastError()) != cudaSuccess) return e;
+    }
+    if (wide && !fused) {
       GemmParams p{};
       p.row0 = c0 + w; p.a_col0 = c0; p.K = w; p.b_row0 = 0; p.b_col0 = 0; p.b_rows_per_job = 256; p.c_col0 = c0;
       p.N = w; p.mode = 1;
@@ -1256,6 +1596,25 @@ cudaError_t tb_chol_tc_factor(float* L32, float* Linv32, void* L16, float* Linv2
       if ((e = gemm(col16 ? tm_x16 : tm_inv256, p)) != cudaSuccess) return e;
     }
     if (mark) mark(mark_ctx, 1, 1);
+    if (fused) {
+      // timed as chol_update: it is the update of these rows (plus the panel product that used to be its own launch)
+      if (mark) mark(mark_ctx, 0, 0);
+      GemmParams p{};
+      p.n_jobs = n_jobs; p.ntp = ntp; p.L32 = L32; p.L16 = static_cast<__half*>(L16);
+      p.row0 = c0 + w; p.row_end = ntp; p.n_mtiles = (ntp - p.row0 + TBM - 1) / TBM;
+      p.K = c0; p.c_col0 = c0; p.N = w; p.from_c = 1; p.fc = *from_c;
+      const int items = n_jobs * p.n_mtiles;
+      const int grid = items < n_sm ? items : n_sm;
+#define TB_FUSED_LAUNCH(S, W) panel_fused_kernel<S, W><<<grid, t_threads(W), F_SMEM, st>>>(tm_l16, tm_x16, p)
+      // (int32 cross-products: eight epilogue warps -- at sixteen, 96 registers per thread do not hold a prefetched unit)
+      if (!from_c->c16) TB_FUSED_LAUNCH(2, 8);
+      else if (epi_warps == 16) TB_FUSED_LAUNCH(1, 16);
+      else TB_FUSED_LAUNCH(1, 8);
+#undef TB_FUSED_LAUNCH
+      launches[0]++;
+      if ((e = cudaGetLastError()) != cudaSuccess) return e;
+      if (mark) mark(mark_ctx, 0, 1);
+    }
   }
   return cudaSuccess;
 }

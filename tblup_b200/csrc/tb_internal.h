@@ -125,6 +125,7 @@ struct TbCtx {
   int chain_fused = -1;           // fused diagonal-block chain (one launch per block column) for waves of at most this many jobs; -1: SM count
   int epi_warps = 16;             // epilogue warps of the Cholesky GEMM kernel (8: round-2 first version)
   int t16 = 1;                    // 1: block-column entries below the diagonal block live as halves in L16 between update and panel GEMM
+  int panel_fused = 1;            // 1: with t16, those entries are updated and finished in one launch without leaving shared memory
   int wide_panel = 1;             // 1: 256-wide panel solve through the inverse of the diagonal block (chol_tc.cu)
   int fuse_scale = 1;             // 1: with one contiguous row set the scaled fp32 matrix is never written by a pass of
                                   //    its own (formed inside the Cholesky updates, or -- fuse_in_gram -- by the Gram epilogue)
@@ -317,7 +318,7 @@ cudaError_t tb_chol_tc_init();
 cudaError_t tb_chol_tc_factor(float* L32, float* Linv32, void* L16, float* Linv256, int* status, int n_jobs, int ntp,
                               int n_sm, cudaStream_t st, int* launches, std::string* err,
                               void (*mark)(void*, int, int), void* mark_ctx, const TbFromC* from_c = nullptr,
-                              int t16 = 1, int epi_warps = 16, int chain_fused_jobs = 0);
+                              int t16 = 1, int epi_warps = 16, int chain_fused_jobs = 0, int panel_fused = 1);
 
 // microbench.cu
 cudaError_t tb_microbench_dmma(int n_sm, cudaStream_t st, double* tflops);

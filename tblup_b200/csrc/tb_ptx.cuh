@@ -62,6 +62,19 @@ __device__ __forceinline__ void tma_load_2d(void* smem_dst, const void* tmap, ui
       : "memory");
 }
 
+// 2-D tiled store from shared memory (same box and swizzle as the tensor map's loads); rows outside the tensor are
+// clipped.  Completion is tracked per thread with bulk groups.
+__device__ __forceinline__ void tma_store_2d(const void* tmap, const void* smem_src, int c0, int c1) {
+  asm volatile("cp.async.bulk.tensor.2d.global.shared::cta.bulk_group [%0, {%2, %3}], [%1];"
+               ::"l"(reinterpret_cast<uint64_t>(tmap)), "r"(smem_u32(smem_src)), "r"(c0), "r"(c1)
+               : "memory");
+}
+__device__ __forceinline__ void bulk_commit_group() { asm volatile("cp.async.bulk.commit_group;" ::: "memory"); }
+// every store committed by this thread has finished READING its shared-memory source (the buffer may be rewritten)
+__device__ __forceinline__ void bulk_wait_group_read0() { asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory"); }
+// every store committed by this thread is complete
+__device__ __forceinline__ void bulk_wait_group0() { asm volatile("cp.async.bulk.wait_group 0;" ::: "memory"); }
+
 // Same, delivered to the same shared-memory offset (and signalled on the same mbarrier offset) of every CTA of the
 // cluster whose bit is set in cta_mask.
 __device__ __forceinline__ void tma_load_2d_multicast(void* smem_dst, const void* tmap, uint64_t* bar, int c0, int c1,
@@ -238,6 +251,16 @@ __device__ __forceinline__ void tmem_ld_32x32(uint32_t taddr, uint32_t (&v)[32])
         "=r"(v[8]), "=r"(v[9]), "=r"(v[10]), "=r"(v[11]), "=r"(v[12]), "=r"(v[13]), "=r"(v[14]), "=r"(v[15]),
         "=r"(v[16]), "=r"(v[17]), "=r"(v[18]), "=r"(v[19]), "=r"(v[20]), "=r"(v[21]), "=r"(v[22]), "=r"(v[23]),
         "=r"(v[24]), "=r"(v[25]), "=r"(v[26]), "=r"(v[27]), "=r"(v[28]), "=r"(v[29]), "=r"(v[30]), "=r"(v[31])
+      : "r"(taddr)
+      : "memory");
+}
+// 32 lanes x 16 consecutive 32-bit columns (half the registers of the x32 form)
+__device__ __forceinline__ void tmem_ld_32x16(uint32_t taddr, uint32_t (&v)[16]) {
+  asm volatile(
+      "tcgen05.ld.sync.aligned.32x32b.x16.b32 "
+      "{%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15}, [%16];"
+      : "=r"(v[0]), "=r"(v[1]), "=r"(v[2]), "=r"(v[3]), "=r"(v[4]), "=r"(v[5]), "=r"(v[6]), "=r"(v[7]),
+        "=r"(v[8]), "=r"(v[9]), "=r"(v[10]), "=r"(v[11]), "=r"(v[12]), "=r"(v[13]), "=r"(v[14]), "=r"(v[15])
       : "r"(taddr)
       : "memory");
 }
