@@ -239,6 +239,26 @@ int tb_knockout(tb_ctx* ctx, const int32_t* genome, int k, int slot, double h2, 
                 uint8_t* keep_out, double* best_fitness_out, int32_t* n_evals_out, int32_t* n_batches_out);
 int tb_knockout_scan(tb_ctx* ctx, const int32_t* genome, int k, int slot, double h2, int mode_rule, double* fitness_out);
 
+/* ---- panel models: marker effects and breeding values (tblup/evaluator.py:284 forms the GBLUP predictions of every
+ * animal and keeps the validation entries; :311-314 fits a Ridge model and discards it after one predict) ------------
+ * tb_fit_effects solves every genome staged with tb_stage_genomes on row set `slot` exactly as tb_eval_staged does
+ * (same branch rule, precision and fp64 fallback; fitness_out [P], nullable, receives the same values) and turns each
+ * solution alpha into one effect per listed marker (flat, staged order, duplicates included):
+ *   centre_q = colsum_q / N (2p over the N frequency animals of the branch),  d = (2 N S - Q) / (2 N^2),
+ *   effect_q = (sum_{a in T} x_{a,q} alpha_a - centre_q sum_{a in T} alpha_a) / d,
+ *   intercept = 0 (gblup) or the mean training phenotype (snp_blup) -- sklearn Ridge's coef_ / intercept_ there.
+ * tb_predict_effects scores animals (original indices of ctx's data set) with P such models, given as the same flat
+ * marker lists (idx_off: P + 1 offsets) and flat centre / effect arrays plus P intercepts:
+ *   out[g * n_animals + b] = intercept_g + sum_q (x_{b,q} - centre_q) effect_q.
+ * It reads only the resident genotypes, so a model fitted on one context scores the animals of any other context
+ * holding the same markers (e.g. newly genotyped animals, created without phenotypes).  Both run in fp64 in a fixed
+ * order: results are identical between the int8 and 2-bit storages and from run to run. */
+int tb_fit_effects(tb_ctx* ctx, int slot, double h2, int mode_rule, double* effects_out, double* centre_out,
+                   double* intercept_out, double* fitness_out);
+int tb_predict_effects(tb_ctx* ctx, const int32_t* idx_flat, const int64_t* idx_off, int P, const double* centre,
+                       const double* effects, const double* intercept, const int32_t* animals, int n_animals,
+                       double* out);
+
 #ifdef __cplusplus
 }
 #endif

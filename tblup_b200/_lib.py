@@ -58,6 +58,10 @@ SYMBOLS = {
     "tb_knockout_scan": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_double, C.c_int, C.c_void_p]),
     "tb_set_stream": (C.c_int, [C.c_void_p, C.c_void_p]),
     "tb_microbench": (C.c_int, [C.c_void_p, C.c_int, C.c_void_p]),
+    "tb_fit_effects": (C.c_int, [C.c_void_p, C.c_int, C.c_double, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p,
+                                 C.c_void_p]),
+    "tb_predict_effects": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p,
+                                     C.c_void_p, C.c_int, C.c_void_p]),
 }
 
 _lib = None

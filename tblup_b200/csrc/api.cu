@@ -141,18 +141,40 @@ void mark_cb(void* p, int which, int end) {
   }
 }
 
-int fp64_fallback(TbCtx* c, const int32_t* slots, int n_slots, double h2, int mode_rule, double* d_fit);
+int fp64_fallback(TbCtx* c, const int32_t* slots, int n_slots, double h2, int mode_rule, double* d_fit, double* d_alpha);
+
+// d_alpha [P][ntp] (one row set): rows [w0, w0 + Wc) <- the solutions of the wave just solved.  Entry i of a job's
+// vector belongs to training animal i of the row set, d_tpos[i], on every layout: the solves index alpha by training
+// position and reach the universe row through tpos (prefix, aligned hole) or through the panel permutation, where
+// d_ident[i] = i is panel row rowmap[d_tpos[i]] = i.  With one row set the arena places the vectors at one stride.
+int copy_alpha(TbCtx* c, double* d_alpha, int w0, int Wc, int ntp) {
+  const std::vector<double*>& al = c->dbg.alpha;
+  const ptrdiff_t stride = Wc > 1 ? al[1] - al[0] : ntp;
+  bool uniform = stride >= ntp;
+  for (int w = 1; w < Wc && uniform; ++w) uniform = al[w] - al[w - 1] == stride;
+  if (uniform) {
+    TB_CUDA(c, cudaMemcpy2DAsync(d_alpha + (size_t)w0 * ntp, (size_t)ntp * sizeof(double), al[0], (size_t)stride * sizeof(double),
+                                 (size_t)ntp * sizeof(double), (size_t)Wc, cudaMemcpyDeviceToDevice, c->stream));
+    return 0;
+  }
+  for (int w = 0; w < Wc; ++w)
+    TB_CUDA(c, cudaMemcpyAsync(d_alpha + (size_t)(w0 + w) * ntp, al[w], (size_t)ntp * sizeof(double),
+                               cudaMemcpyDeviceToDevice, c->stream));
+  return 0;
+}
 
 struct SlotView {
   const TbRowSet* rs;
   size_t m_elems, linv_elems;
 };
 
+// d_alpha (nullable, one row set only): [P][ntp] device destination of every genome's solution (see copy_alpha)
 int eval_core(TbCtx* c, const int32_t* slots, int n_slots, double h2, int mode_rule, double* d_fit,
-              bool allow_fallback = true) {
+              bool allow_fallback = true, double* d_alpha = nullptr) {
   const auto t_host0 = std::chrono::steady_clock::now();
   if (c->P <= 0) return fail(c, "tb_eval_staged: no genomes staged");
   if (n_slots <= 0 || n_slots > TB_MAX_SLOTS) return fail(c, "tb_eval_staged: bad n_slots");
+  if (d_alpha && n_slots != 1) return fail(c, "internal: solutions are kept for one row set only");
   if (!(h2 > 0.0) || !(h2 <= 1.0)) return fail(c, "tb_eval_staged: heritability must be in (0, 1]");
   if (mode_rule < 0 || mode_rule > 2) return fail(c, "tb_eval_staged: bad mode_rule");
   const double lambda = (1.0 - h2) / h2;   // tblup/evaluator.py:277
@@ -552,6 +574,8 @@ int eval_core(TbCtx* c, const int32_t* slots, int n_slots, double h2, int mode_r
                                        c->solve_pair));
       span_end(c, sp);
       count(c, TB_ST_SOLVE, 1);
+      if (d_alpha)
+        if (int rc = copy_alpha(c, d_alpha, w0, Wc, max_ntp)) return rc;
       continue;
     }
 
@@ -584,11 +608,13 @@ int eval_core(TbCtx* c, const int32_t* slots, int n_slots, double h2, int mode_r
     TB_CUDA(c, tb_launch_solve(d_solve, n_jobs, max_ntp, st));
     span_end(c, sp);
     count(c, TB_ST_SOLVE, 1);
+    if (d_alpha)
+      if (int rc = copy_alpha(c, d_alpha, w0, Wc, max_ntp)) return rc;
   }
   // host time spent issuing the evaluation (everything above is asynchronous): diagnostics, "last_issue_us"
   c->last_issue_us = (long long)std::chrono::duration_cast<std::chrono::microseconds>(
                          std::chrono::steady_clock::now() - t_host0).count();
-  if (mixed && allow_fallback && c->stop_after < 0 && !c->no_fallback) return fp64_fallback(c, slots, n_slots, h2, mode_rule, d_fit);
+  if (mixed && allow_fallback && c->stop_after < 0 && !c->no_fallback) return fp64_fallback(c, slots, n_slots, h2, mode_rule, d_fit, d_alpha);
   return 0;
 }
 
@@ -596,7 +622,7 @@ int eval_core(TbCtx* c, const int32_t* slots, int n_slots, double h2, int mode_r
 // refinement: lambda -> 0, i.e. h2 -> 1, makes A ill-conditioned) are evaluated again with the fp64 Cholesky, which
 // is what the reference's fp64 inverse (tblup/evaluator.py:282) can still handle.  One small D2H of the flags per
 // evaluation; in the normal case nothing else happens.
-int fp64_fallback(TbCtx* c, const int32_t* slots, int n_slots, double h2, int mode_rule, double* d_fit) {
+int fp64_fallback(TbCtx* c, const int32_t* slots, int n_slots, double h2, int mode_rule, double* d_fit, double* d_alpha) {
   const int P = c->P;
   std::vector<int> h_fail((size_t)P * n_slots);
   TB_CUDA(c, cudaMemcpyAsync(h_fail.data(), c->d_fail, h_fail.size() * sizeof(int), cudaMemcpyDeviceToHost, c->stream));
@@ -617,9 +643,13 @@ int fp64_fallback(TbCtx* c, const int32_t* slots, int n_slots, double h2, int mo
   for (size_t j = 0; j < redo.size(); ++j) sub_off[j + 1] = sub_off[j] + (c->h_off[redo[j] + 1] - c->h_off[redo[j]]);
   int* d_sub = nullptr;
   double* d_subfit = nullptr;
+  double* d_subalpha = nullptr;                      // [redo][ntp] solutions of the sub-batch (kept alpha only)
+  const int ntp = d_alpha ? c->slots[slots[0]].ntp : 0;
   TB_CUDA(c, cudaMalloc(&d_sub, (size_t)sub_off.back() * sizeof(int)));
-  if (cudaMalloc(&d_subfit, redo.size() * n_slots * sizeof(double)) != cudaSuccess) {
+  if (cudaMalloc(&d_subfit, redo.size() * n_slots * sizeof(double)) != cudaSuccess ||
+      (d_alpha && cudaMalloc(&d_subalpha, redo.size() * ntp * sizeof(double)) != cudaSuccess)) {
     cudaFree(d_sub);
+    cudaFree(d_subfit);
     return fail(c, "fp64 fallback: out of memory", -2);
   }
   for (size_t j = 0; j < redo.size(); ++j)
@@ -637,7 +667,7 @@ int fp64_fallback(TbCtx* c, const int32_t* slots, int n_slots, double h2, int mo
   c->idx_cap = (size_t)sub_off.back();
   c->P = (int)redo.size();
   c->precision = 1;
-  int rc = eval_core(c, slots, n_slots, h2, mode_rule, d_subfit, false);
+  int rc = eval_core(c, slots, n_slots, h2, mode_rule, d_subfit, false, d_subalpha);
   c->precision = keep_prec;
   c->P = keep_P;
   c->d_idx = keep_idx;
@@ -654,10 +684,15 @@ int fp64_fallback(TbCtx* c, const int32_t* slots, int n_slots, double h2, int mo
         if (h_fail[(size_t)redo[j] * n_slots + s])
           cudaMemcpyAsync(d_fit + (size_t)redo[j] * n_slots + s, d_subfit + j * n_slots + s, sizeof(double),
                           cudaMemcpyDeviceToDevice, c->stream);
+    if (d_alpha)                                     // one row set: every redone genome failed on it
+      for (size_t j = 0; j < redo.size(); ++j)
+        cudaMemcpyAsync(d_alpha + (size_t)redo[j] * ntp, d_subalpha + j * ntp, (size_t)ntp * sizeof(double),
+                        cudaMemcpyDeviceToDevice, c->stream);
   }
   cudaError_t se = cudaStreamSynchronize(c->stream);
   cudaFree(d_sub);
   cudaFree(d_subfit);
+  cudaFree(d_subalpha);
   if (rc) return rc;
   if (se != cudaSuccess) return fail(c, std::string("fp64 fallback: ") + cudaGetErrorString(se), -2);
   c->last_fallbacks = n_failed;
@@ -668,6 +703,9 @@ int fp64_fallback(TbCtx* c, const int32_t* slots, int n_slots, double h2, int mo
 
 int tb_internal_eval_device(TbCtx* c, const int32_t* slots, int n_slots, double h2, int mode_rule, double* d_fit) {
   return eval_core(c, slots, n_slots, h2, mode_rule, d_fit);
+}
+int tb_internal_eval_alpha(TbCtx* c, int slot, double h2, int mode_rule, double* d_fit, double* d_alpha) {
+  return eval_core(c, &slot, 1, h2, mode_rule, d_fit, true, d_alpha);
 }
 void tb_internal_collect_spans(TbCtx* c) { spans_collect(c); }
 
@@ -1023,6 +1061,7 @@ int tb_set_rowset(tb_ctx* c, int slot, const int32_t* train, int n_t, const int3
     mean += yt[i];
   }
   mean /= n_t;
+  r.yt_mean = mean;
   for (int i = 0; i < n_t; ++i) ytc[i] = yt[i] - mean;
   for (int i = 0; i < n_v; ++i) yv[i] = c->y_univ[vpos[i]];
   TB_CUDA(c, cudaMalloc(&r.d_tpos, n_t * sizeof(int)));

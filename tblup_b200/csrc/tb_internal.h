@@ -42,6 +42,7 @@ struct TbRowSet {
   double* d_yt_raw = nullptr;   // [ntp] (zero padded)
   double* d_yt_ctr = nullptr;   // [ntp] y_t minus its mean
   double* d_yv = nullptr;       // [n_v]
+  double yt_mean = 0.0;         // mean phenotype of the training animals (intercept of the snp_blup model)
   std::vector<unsigned char> has_train;   // per 128-row universe block: contains a training animal
   bool contiguous = false;      // training animal b sits at universe position b
   // "contiguous with one hole": training animal i sits at i for i < hole0 and at i + gap beyond (hole0, gap multiples
@@ -327,5 +328,8 @@ cudaError_t tb_microbench_umma(int which, int n_sm, cudaStream_t st, double* top
 // api.cu internals used by de.cu: evaluate the genomes already staged on the device (c->d_idx, c->h_off, c->P)
 // into a device buffer [P * n_slots] (asynchronous on c->stream), and fold the profiling spans after a sync.
 int tb_internal_eval_device(TbCtx* c, const int32_t* slots, int n_slots, double h2, int mode_rule, double* d_fit);
+// the same on ONE row set, also writing every genome's solution: d_alpha [P][ntp of the row set], entry i of genome g
+// belonging to the training animal at d_tpos[i] of the row set (entries beyond n_t are padding) -- used by tb_fit_effects
+int tb_internal_eval_alpha(TbCtx* c, int slot, double h2, int mode_rule, double* d_fit, double* d_alpha);
 void tb_internal_collect_spans(TbCtx* c);
 void tb_de_release(TbCtx* c);

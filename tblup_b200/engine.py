@@ -77,10 +77,12 @@ def pack_genomes(genomes, n_markers):
 class GblupEngine:
     """One data set on one GPU.  Not thread-safe (one host thread per context, like the C-ABI)."""
 
-    def __init__(self, geno, pheno, perm=None, device=0, storage="packed2"):
+    def __init__(self, geno, pheno=None, perm=None, device=0, storage="packed2"):
         """``geno``: dense dosages (animals x markers, any real dtype holding 0/1/2) or a
         ``genoio.PackedGenotypes``; ``storage``: how the matrix stays resident in HBM, ``"int8"`` (one byte per
-        dosage) or ``"packed2"`` (2 bits per dosage, a quarter of the bytes; same results bit for bit)."""
+        dosage) or ``"packed2"`` (2 bits per dosage, a quarter of the bytes; same results bit for bit).
+        ``pheno=None``: a context without phenotypes, which only scores animals with models fitted elsewhere
+        (``predict``); row sets, evaluations and fits are refused on it."""
         from .genoio import PackedGenotypes
         self._lib = _lib.load()
         self._ctx = C.c_void_p()
@@ -91,6 +93,9 @@ class GblupEngine:
         else:
             g, layout = as_dosage_int8(geno), LAYOUT_INT8_ANIMAL_MAJOR
             shape = g.shape
+        self.has_phenotypes = pheno is not None
+        if pheno is None:
+            pheno = np.zeros(shape[0])
         y = np.ascontiguousarray(np.asarray(pheno, dtype=np.float64).ravel())
         if y.shape[0] != shape[0]:
             raise ValueError("phenotype vector has %d entries for %d animals" % (y.shape[0], shape[0]))
@@ -121,6 +126,7 @@ class GblupEngine:
             other._ctx = C.c_void_p()
             raise RuntimeError("tb_clone failed (%d): %s" % (rc, self._lib.tb_last_error(None).decode()))
         other.n, other.m, other.storage, other.device, other._n_staged = self.n, self.m, self.storage, int(device), 0
+        other.has_phenotypes = self.has_phenotypes
         return other
 
     def close(self):
@@ -146,6 +152,8 @@ class GblupEngine:
 
     # -- configuration -------------------------------------------------------------------------
     def set_rowset(self, slot, train, valid):
+        if not self.has_phenotypes:
+            raise RuntimeError("this context holds no phenotypes: it can only score animals (predict)")
         t = np.ascontiguousarray(np.asarray(train, dtype=np.int32))
         v = np.ascontiguousarray(np.asarray(valid, dtype=np.int32))
         self._check(self._lib.tb_set_rowset(self._ctx, int(slot), t.ctypes.data, t.size, v.ctypes.data, v.size),
@@ -191,6 +199,45 @@ class GblupEngine:
         self._check(self._lib.tb_eval(self._ctx, s.ctypes.data, s.size, flat.ctypes.data, off.ctypes.data, P,
                                       float(h2), int(mode), out.ctypes.data), "tb_eval")
         self._n_staged = P
+        return out
+
+    # -- panel models: marker effects and breeding values -----------------------------------------
+    def fit_models(self, genomes, slot=0, h2=0.4, mode=MODE_AUTO):
+        """One ``PanelModel`` per genome, trained on row set ``slot`` exactly as the fitness is computed there (same
+        branch rule, precision and fp64 fallback; each model's ``fitness`` is the value ``evaluate`` returns).  The
+        genomes become the staged batch (``stage``)."""
+        from .model import PanelModel
+        flat, off = pack_genomes(genomes, self.m)
+        self.stage(flat=flat, off=off)
+        P = off.size - 1
+        effects = np.empty(flat.size, dtype=np.float64)
+        centre = np.empty(flat.size, dtype=np.float64)
+        intercept = np.empty(P, dtype=np.float64)
+        fitness = np.empty(P, dtype=np.float64)
+        self._check(self._lib.tb_fit_effects(self._ctx, int(slot), float(h2), int(mode), effects.ctypes.data,
+                                             centre.ctypes.data, intercept.ctypes.data, fitness.ctypes.data),
+                    "tb_fit_effects")
+        models = []
+        for i in range(P):
+            a, b = int(off[i]), int(off[i + 1])
+            k = b - a
+            gblup = mode == MODE_GBLUP or (mode == MODE_AUTO and k > self.n)
+            models.append(PanelModel(flat[a:b], centre[a:b], effects[a:b], intercept[i],
+                                     "gblup" if gblup else "snp_blup", h2, fitness[i]))
+        return models
+
+    def predict(self, models, animals):
+        """Breeding values of ``animals`` (original indices of this context's data set) under each model:
+        array (len(models), len(animals)).  The models may come from another context holding the same markers."""
+        flat, off = pack_genomes([mdl.markers for mdl in models], self.m)
+        centre = np.ascontiguousarray(np.concatenate([mdl.centre for mdl in models]), dtype=np.float64)
+        effects = np.ascontiguousarray(np.concatenate([mdl.effects for mdl in models]), dtype=np.float64)
+        intercept = np.ascontiguousarray([mdl.intercept for mdl in models], dtype=np.float64)
+        a = np.ascontiguousarray(np.asarray(animals, dtype=np.int32).ravel())
+        out = np.empty((len(models), a.size), dtype=np.float64)
+        self._check(self._lib.tb_predict_effects(self._ctx, flat.ctypes.data, off.ctypes.data, len(models),
+                                                 centre.ctypes.data, effects.ctypes.data, intercept.ctypes.data,
+                                                 a.ctypes.data, a.size, out.ctypes.data), "tb_predict_effects")
         return out
 
     # -- per-marker statistics (top-SNPs seeder, tblup/seeder.py:144-160) ------------------------

@@ -304,6 +304,29 @@ class BlupParallelEvaluator(ParallelEvaluator):
         return [float(v) for v in self._fitness_matrix(genomes, [TESTING_SLOT])[:, 0]]
 
 
+    # ---- panel models (the model behind evaluate_testing's number) ----------------------------------------------
+    def _testing_genome(self, genome):
+        if self.snp_remover is None:
+            return np.asarray(genome).astype(int)
+        return self.snp_remover.combine_with_removed(genome)
+
+    def fit_model(self, genome):
+        """The ``PanelModel`` whose testing accuracy ``evaluate_testing`` reports: trained on training + validation
+        (the testing row set), on the genome united with every SNP removed so far, on the first engine."""
+        if len(self.consumers) == 0:
+            raise AttributeError("Workers are not set up.")
+        return self.consumers[0].fit_models([self._testing_genome(genome)], slot=TESTING_SLOT, h2=self.h2,
+                                            mode=MODE_AUTO)[0]
+
+    def breeding_values(self, genome, animals=None):
+        """Genomic estimated breeding values under ``fit_model(genome)`` of ``animals`` (original indices; default:
+        the testing animals, whose |Pearson r| with the phenotypes is the testing accuracy)."""
+        model = self.fit_model(genome)
+        if animals is None:
+            animals = self.testing_indices
+        return self.consumers[0].predict([model], animals)[0]
+
+
 class InterGCVBlupParallelEvaluator(BlupParallelEvaluator):
     """Validation fold rotates with the generation (evaluator.py:434-491)."""
 
