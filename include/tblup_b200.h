@@ -54,7 +54,8 @@ const char* tb_last_error(const tb_ctx* ctx);
 
 /* Upload a data set once.  Takes over `np.load(data_path)` / `np.load(labels_path)` of every worker
  * (tblup/evaluator.py:215-216).  geno: [n][m] dosages in {0,1,2}, animal-major (the .npy layout);
- * y: [n]; perm: [n] or NULL, animal stored at "universe" position p is perm[p] (put the animals the
+ * y: [n], or NULL for a context without phenotypes (it only scores animals with tb_predict_effects; row sets and
+ * everything built on them are refused); perm: [n] or NULL, animal stored at "universe" position p is perm[p] (put the animals the
  * fitness reads first: training, validation, testing -- the Gram then only covers that prefix). */
 int tb_create(const int8_t* geno, int n, int m, const double* y, const int32_t* perm, int device, tb_ctx** out);
 
@@ -258,6 +259,36 @@ int tb_fit_effects(tb_ctx* ctx, int slot, double h2, int mode_rule, double* effe
 int tb_predict_effects(tb_ctx* ctx, const int32_t* idx_flat, const int64_t* idx_off, int P, const double* centre,
                        const double* effects, const double* intercept, const int32_t* animals, int n_animals,
                        double* out);
+
+/* ---- REML heritability: the restricted log-likelihood of a panel's genomic model as a profile in h2 ---------------
+ * For a genome (marker list j_1..j_k, duplicates count twice) and row set `slot` with training animals T, n = n_t:
+ *
+ *     y_T = 1 mu + g + e,   g ~ N(0, sigma_g^2 G_TT),   e ~ N(0, sigma_e^2 I),   h2 = sigma_g^2 / (sigma_g^2 + sigma_e^2),   lambda = (1 - h2)/h2
+ *
+ * Here G_TT is exactly the matrix the fitness factors for that genome on that row set.  The same branch rule
+ * (mode_rule, TB_MODE_AUTO: k > n -> gblup) picks the frequency animals: all n animals for gblup, the training animals
+ * for snp_blup.  y_T is the raw training phenotype.  The intercept mu is a fixed effect of the model, so centring y
+ * changes nothing.  With A = G_TT + lambda I = L L^T, u = L^-1 1 and v = L^-1 y_T:
+ *
+ *     a = u'u,  b = u'v,  c = v'v,  mu^ = b/a,  q = c - b^2/a,  sigma_g^2^ = q/(n - 1),  sigma_e^2^ = lambda sigma_g^2^
+ *     l(h2) = -1/2 [ (n - 1)(log(2 pi sigma_g^2^) + 1) + log|A| + log a ],   log|A| = 2 sum_i log L_ii
+ *
+ * This is the restricted log-likelihood -1/2[log|V| + log|X'V^-1 X| + y'Py] - ((n-1)/2) log 2 pi with X = 1 and
+ * V = sigma_g^2 A, maximised over sigma_g^2 in closed form.  So l is a one-dimensional profile in h2.  Padding rows of
+ * the factor (identity) add 0 to log|A| and to every quadratic form.  For snp_blup, G_TT 1 = 0, so a = n/lambda.  The
+ * formula needs no special case.
+ *
+ * tb_reml_profile evaluates l, sigma_g^2^ and mu^ for every genome staged with tb_stage_genomes at n_h2 points each:
+ * h2 is one list of n_h2 values shared by every genome (per_genome = 0) or [P][n_h2] (per_genome != 0); the outputs
+ * are host [P][n_h2], sigma_g2_out and mu_out may be NULL.  All points of a genome share its gather, centring terms
+ * and Gram (64 points per pass); every point gets its own fp64 A and fp64 Cholesky, whatever the `precision` option
+ * says (a determinant cannot be refined).  Results are identical between the storages and from run to run; a job
+ * whose factorisation meets a non-positive pivot returns NaN in all three outputs.  Refused, with a tb_last_error
+ * message: an h2 outside (0, 1), n_h2 < 1, an undefined row set, a context created without phenotypes, an empty
+ * genome.  The context's options and its last-evaluation facts (tb_get_info "last_*") are unchanged afterwards; the
+ * staged batch stays staged. */
+int tb_reml_profile(tb_ctx* ctx, int slot, int mode_rule, const double* h2, int n_h2, int per_genome,
+                    double* loglik_out, double* sigma_g2_out, double* mu_out);
 
 #ifdef __cplusplus
 }

@@ -62,6 +62,8 @@ SYMBOLS = {
                                  C.c_void_p]),
     "tb_predict_effects": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p,
                                      C.c_void_p, C.c_int, C.c_void_p]),
+    "tb_reml_profile": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_void_p,
+                                  C.c_void_p]),
 }
 
 _lib = None

@@ -169,13 +169,16 @@ struct SlotView {
 };
 
 // d_alpha (nullable, one row set only): [P][ntp] device destination of every genome's solution (see copy_alpha)
+// reml (nullable): the "row sets" are reml->n copies of one row set, one per h2 point of the profile; each job gets its
+// own lambda, an fp64 A of ntp x ntp only (no G_vt rows) and reml_kernel instead of the solve (d_fit and h2 unused)
 int eval_core(TbCtx* c, const int32_t* slots, int n_slots, double h2, int mode_rule, double* d_fit,
-              bool allow_fallback = true, double* d_alpha = nullptr) {
+              bool allow_fallback = true, double* d_alpha = nullptr, const TbRemlReq* reml = nullptr) {
   const auto t_host0 = std::chrono::steady_clock::now();
   if (c->P <= 0) return fail(c, "tb_eval_staged: no genomes staged");
   if (n_slots <= 0 || n_slots > TB_MAX_SLOTS) return fail(c, "tb_eval_staged: bad n_slots");
   if (d_alpha && n_slots != 1) return fail(c, "internal: solutions are kept for one row set only");
-  if (!(h2 > 0.0) || !(h2 <= 1.0)) return fail(c, "tb_eval_staged: heritability must be in (0, 1]");
+  if (reml && (d_alpha || reml->n != n_slots)) return fail(c, "internal: bad REML request");
+  if (!reml && (!(h2 > 0.0) || !(h2 <= 1.0))) return fail(c, "tb_eval_staged: heritability must be in (0, 1]");
   if (mode_rule < 0 || mode_rule > 2) return fail(c, "tb_eval_staged: bad mode_rule");
   const double lambda = (1.0 - h2) / h2;   // tblup/evaluator.py:277
   std::vector<SlotView> sv(n_slots);
@@ -187,14 +190,15 @@ int eval_core(TbCtx* c, const int32_t* slots, int n_slots, double h2, int mode_r
       return fail(c, "tb_eval_staged: row set " + std::to_string(slots[s]) + " is not defined");
     const TbRowSet* rs = &c->slots[slots[s]];
     sv[s].rs = rs;
-    sv[s].m_elems = (size_t)(rs->ntp + rs->n_v) * rs->ntp;
+    const int n_v = reml ? 0 : rs->n_v;              // REML forms A only
+    sv[s].m_elems = (size_t)(rs->ntp + n_v) * rs->ntp;
     sv[s].linv_elems = (size_t)rs->ntp * TB_NB;
     rpad = std::max(rpad, rs->rpad);
     max_ntp = std::max(max_ntp, rs->ntp);
-    max_rows = std::max(max_rows, rs->ntp + rs->n_v);
+    max_rows = std::max(max_rows, rs->ntp + n_v);
     if (has_train.size() < rs->has_train.size()) has_train.resize(rs->has_train.size(), 0);
     for (size_t i = 0; i < rs->has_train.size(); ++i) has_train[i] |= rs->has_train[i];
-    per_ind += (sv[s].m_elems + sv[s].linv_elems + rs->ntp + rs->n_v) * sizeof(double) + 1024;
+    per_ind += (sv[s].m_elems + sv[s].linv_elems + rs->ntp + n_v) * sizeof(double) + (reml ? sizeof(TbRemlJob) : 0) + 1024;
   }
   has_train.resize(rpad / TB_GRAM_BM, 0);
   const int P = c->P;
@@ -210,7 +214,7 @@ int eval_core(TbCtx* c, const int32_t* slots, int n_slots, double h2, int mode_r
   c->last_fp4 = fp4 ? 1 : 0;
   // a single scattered row set (Monte-Carlo split, unaligned fold, custom splitter): permute the panel rows at gather
   // time -- training animals first, validation animals next -- and everything downstream sees a plain prefix
-  if (n_slots > 1 && c->perm_rows && fp4 && c->precision == 0 && c->stop_after < 0) {
+  if (n_slots > 1 && !reml && c->perm_rows && fp4 && c->precision == 0 && c->stop_after < 0) {
     // Several row sets share one Gram only while each of them can run the contiguous kernels (a prefix, or -- int16
     // layout -- a prefix with one aligned hole).  Otherwise the refinement would fall back to per-element position
     // lookups (measured 14x slower per solve than a whole extra Gram): evaluate the row sets one at a time instead,
@@ -244,7 +248,7 @@ int eval_core(TbCtx* c, const int32_t* slots, int n_slots, double h2, int mode_r
     }
   }
   if (n_slots > 1) c->last_split = 0;
-  const bool use_perm = n_slots == 1 && c->perm_rows && fp4 && !sv[0].rs->contiguous && sv[0].rs->perm_ok;
+  const bool use_perm = (n_slots == 1 || reml) && c->perm_rows && fp4 && !sv[0].rs->contiguous && sv[0].rs->perm_ok;
   c->last_perm = use_perm ? 1 : 0;
   if (use_perm) {
     const TbRowSet* rs = sv[0].rs;
@@ -253,7 +257,8 @@ int eval_core(TbCtx* c, const int32_t* slots, int n_slots, double h2, int mode_r
     for (int blk = 0; blk * TB_GRAM_BM < rs->n_t; ++blk) has_train[blk] = 1;
   }
   // the mixed path turns cross-products (<= 4 k) into floats through the 2^23 mantissa trick: 4 kmax < 2^23
-  bool mixed = c->precision == 0 && tb_solve_mixed_fits(max_ntp) && 4LL * kmax < (1LL << 23);
+  // (REML always runs the fp64 Cholesky: the 10-bit factor would put an error of order n 1e-3 into log|A|)
+  bool mixed = !reml && c->precision == 0 && tb_solve_mixed_fits(max_ntp) && 4LL * kmax < (1LL << 23);
   for (int s = 0; s < n_slots; ++s) mixed = mixed && sv[s].rs->ntp == max_ntp;
   c->last_mixed = mixed ? 1 : 0;
   if (allow_fallback) c->last_fallbacks = 0;
@@ -305,6 +310,7 @@ int eval_core(TbCtx* c, const int32_t* slots, int n_slots, double h2, int mode_r
   int W = (int)std::min<long long>(Wll, P);
   if (c->max_wave > 0) W = std::min(W, c->max_wave);
   W = std::max(1, std::min(W, 1024));
+  if (reml) W = std::max(1, std::min(W, 65535 / n_slots));   // jobs of a wave index gridDim.y of the Cholesky GEMMs
   c->last_wave = W;
   if (int rc = ensure_ws(c, fixed + per_ind * (size_t)W)) return rc;
 
@@ -330,6 +336,7 @@ int eval_core(TbCtx* c, const int32_t* slots, int n_slots, double h2, int mode_r
   std::vector<TbSolveMixedJob> h_msolve;
   std::vector<const int*> h_cs;
   std::vector<int> h_kb;
+  std::vector<TbRemlJob> h_reml;
 
   for (int w0 = 0; w0 < P; w0 += W) {
     const int Wc = std::min(W, P - w0);
@@ -358,6 +365,7 @@ int eval_core(TbCtx* c, const int32_t* slots, int n_slots, double h2, int mode_r
     TbSolveJob* d_solve = ar.take<TbSolveJob>(n_jobs);
     TbSolveMixedJob* d_msolve = ar.take<TbSolveMixedJob>(n_jobs);
     int* d_sweeps = ar.take<int>(n_jobs);
+    TbRemlJob* d_reml = reml ? ar.take<TbRemlJob>(n_jobs) : nullptr;
     float* d_L32 = nullptr;
     float* d_Linv32 = nullptr;
     unsigned short* d_L16 = nullptr;
@@ -380,6 +388,7 @@ int eval_core(TbCtx* c, const int32_t* slots, int n_slots, double h2, int mode_r
     h_solve.resize(n_jobs);
     h_msolve.resize(n_jobs);
     h_cs.resize(n_jobs);
+    if (reml) h_reml.resize(n_jobs);
     c->dbg.L32 = d_L32;
     c->dbg.L16 = d_L16;
     c->dbg.sweeps = d_sweeps;
@@ -403,19 +412,30 @@ int eval_core(TbCtx* c, const int32_t* slots, int n_slots, double h2, int mode_r
       const int k = (int)(c->h_off[w0 + w + 1] - c->h_off[w0 + w]);
       wave_all_gblup = wave_all_gblup && (mode_rule == TB_MODE_GBLUP || (mode_rule == TB_MODE_AUTO && k > c->n));
     }
-    const int centre_slots = wave_all_gblup ? 1 : n_slots;
-    c->dbg.centre_shared = wave_all_gblup ? 1 : 0;
+    // (the REML jobs of a genome all sit on one row set: one set of terms per genome whatever the branch)
+    const bool centre_shared = wave_all_gblup || reml;
+    const int centre_slots = centre_shared ? 1 : n_slots;
+    c->dbg.centre_shared = centre_shared ? 1 : 0;
     for (int w = 0; w < Wc; ++w) {
       const int k = (int)(c->h_off[w0 + w + 1] - c->h_off[w0 + w]);
       const bool gblup = mode_rule == TB_MODE_GBLUP || (mode_rule == TB_MODE_AUTO && k > c->n);
       for (int s = 0; s < n_slots; ++s) {
         const int job = w * n_slots + s;
-        const int cjob = wave_all_gblup ? w : job;      // index of this job's centring terms
+        const int cjob = centre_shared ? w : job;       // index of this job's centring terms
         const TbRowSet* rs = sv[s].rs;
+        const int n_v = reml ? 0 : rs->n_v;
         double* Mj = mixed ? nullptr : ar.take<double>(sv[s].m_elems);
         double* Lj = mixed ? nullptr : ar.take<double>(sv[s].linv_elems);
         double* aj = ar.take<double>(rs->ntp);
-        double* pj = ar.take<double>(rs->n_v);
+        double* pj = ar.take<double>(n_v);
+        double lambda_j = lambda;
+        if (reml) {
+          const double h2j = reml->h2[(size_t)(w0 + w) * reml->ld + reml->s0 + s];
+          lambda_j = (1.0 - h2j) / h2j;
+          const size_t o = (size_t)(w0 + w) * reml->n_out + reml->s0 + s;
+          h_reml[job] = TbRemlJob{Mj, Lj, rs->d_yt_ctr, d_status + job, rs->yt_mean, rs->n_t, rs->ntp,
+                                  reml->d_loglik + o, reml->d_sigma_g2 + o, reml->d_mu + o};
+        }
         h_cs[cjob] = gblup ? c->d_colsum_all : rs->d_colsum_train;
         TbScaleJob& sj = h_scale[job];
         sj.C = c16 ? reinterpret_cast<const int32_t*>(reinterpret_cast<const int16_t*>(d_C) + (size_t)w * rpad * rpad)
@@ -427,10 +447,10 @@ int eval_core(TbCtx* c, const int32_t* slots, int n_slots, double h2, int mode_r
         sj.M = Mj;
         sj.N = gblup ? c->n : rs->n_t;
         sj.n_t = rs->n_t;
-        sj.n_v = rs->n_v;
+        sj.n_v = n_v;
         sj.ntp = rs->ntp;
         sj.rpad = rpad;
-        sj.lambda = lambda;
+        sj.lambda = lambda_j;
         sj.hole0 = use_perm ? rs->n_t : rs->hole0;
         sj.gap = use_perm ? 0 : rs->gap;
         sj.cw = w;
@@ -447,9 +467,9 @@ int eval_core(TbCtx* c, const int32_t* slots, int n_slots, double h2, int mode_r
         oj.status = d_status + job;
         oj.alpha = aj;
         oj.pred = pj;
-        oj.fitness = d_fit + (size_t)(w0 + w) * n_slots + s;
+        oj.fitness = d_fit ? d_fit + (size_t)(w0 + w) * n_slots + s : nullptr;
         oj.n_t = rs->n_t;
-        oj.n_v = rs->n_v;
+        oj.n_v = n_v;
         oj.ntp = rs->ntp;
         TbSolveMixedJob& mj = h_msolve[job];
         mj.L32 = d_L32 ? d_L32 + (size_t)job * max_ntp * max_ntp : nullptr;
@@ -482,7 +502,7 @@ int eval_core(TbCtx* c, const int32_t* slots, int n_slots, double h2, int mode_r
         c->dbg.alpha[job] = aj;
         c->dbg.pred[job] = pj;
         c->dbg.ntp[job] = rs->ntp;
-        c->dbg.n_v[job] = rs->n_v;
+        c->dbg.n_v[job] = n_v;
       }
     }
     if (ar.off > ar.cap) return fail(c, "internal: wave workspace overflow");
@@ -494,6 +514,7 @@ int eval_core(TbCtx* c, const int32_t* slots, int n_slots, double h2, int mode_r
     TB_CUDA(c, cudaMemcpyAsync(d_chol, h_chol.data(), n_jobs * sizeof(TbCholJob), cudaMemcpyHostToDevice, st));
     TB_CUDA(c, cudaMemcpyAsync(d_solve, h_solve.data(), n_jobs * sizeof(TbSolveJob), cudaMemcpyHostToDevice, st));
     TB_CUDA(c, cudaMemcpyAsync(d_msolve, h_msolve.data(), n_jobs * sizeof(TbSolveMixedJob), cudaMemcpyHostToDevice, st));
+    if (reml) TB_CUDA(c, cudaMemcpyAsync(d_reml, h_reml.data(), n_jobs * sizeof(TbRemlJob), cudaMemcpyHostToDevice, st));
     TB_CUDA(c, cudaMemsetAsync(d_status, 0, n_jobs * sizeof(int), st));
     span_end(c, sp);
 
@@ -605,6 +626,12 @@ int eval_core(TbCtx* c, const int32_t* slots, int n_slots, double h2, int mode_r
     if (c->stop_after == TB_ST_CHOL_UPDATE || c->stop_after == TB_ST_CHOL_PANEL) continue;
 
     sp = span_begin(c, TB_ST_SOLVE);
+    if (reml) {                                      // log|A|, the forward substitution of [y_T, 1] and the profile
+      TB_CUDA(c, tb_launch_reml(d_reml, n_jobs, max_ntp, st));
+      span_end(c, sp);
+      count(c, TB_ST_SOLVE, 1);
+      continue;
+    }
     TB_CUDA(c, tb_launch_solve(d_solve, n_jobs, max_ntp, st));
     span_end(c, sp);
     count(c, TB_ST_SOLVE, 1);
@@ -707,6 +734,11 @@ int tb_internal_eval_device(TbCtx* c, const int32_t* slots, int n_slots, double 
 int tb_internal_eval_alpha(TbCtx* c, int slot, double h2, int mode_rule, double* d_fit, double* d_alpha) {
   return eval_core(c, &slot, 1, h2, mode_rule, d_fit, true, d_alpha);
 }
+int tb_internal_eval_reml(TbCtx* c, int slot, int mode_rule, const TbRemlReq* req) {
+  if (!req || req->n < 1 || req->n > TB_MAX_SLOTS) return fail(c, "internal: bad REML request");
+  const std::vector<int32_t> slots(req->n, slot);
+  return eval_core(c, slots.data(), req->n, 0.0, mode_rule, nullptr, false, nullptr, req);
+}
 void tb_internal_collect_spans(TbCtx* c) { spans_collect(c); }
 
 extern "C" {
@@ -723,7 +755,7 @@ int tb_create_ex(const void* geno_any, int layout, int storage, int n, int m, co
                  int device, tb_ctx** out) {
   if (!out) return -1;
   *out = nullptr;
-  if (!geno_any || !y || n <= 0 || m <= 0) {
+  if (!geno_any || n <= 0 || m <= 0) {
     g_create_err = "tb_create: null or empty input";
     return -1;
   }
@@ -770,8 +802,10 @@ int tb_create_ex(const void* geno_any, int layout, int storage, int n, int m, co
     if (p[i] < 0 || p[i] >= n || c->pos_of[p[i]] != -1) return bail("tb_create: perm is not a permutation of 0..n-1");
     c->pos_of[p[i]] = i;
   }
-  c->y_univ.resize(n);
-  for (int i = 0; i < n; ++i) c->y_univ[i] = y[p[i]];
+  c->has_pheno = y != nullptr;
+  c->y_univ.assign(n, 0.0);
+  if (y)
+    for (int i = 0; i < n; ++i) c->y_univ[i] = y[p[i]];
 
   auto chk = [&](cudaError_t ce, const char* what) {
     if (ce == cudaSuccess) return false;
@@ -891,7 +925,7 @@ int tb_create_ex(const void* geno_any, int layout, int storage, int n, int m, co
   if (chk(tb_gram_tc_init(), "gram kernel init") || chk(tb_chol_init(), "cholesky kernel init") ||
       chk(tb_solve_init(), "solve kernel init") ||
       chk(tb_chol_tc_init(), "tensor-core cholesky init") || chk(tb_solve_mixed_init(), "mixed solve init") ||
-      chk(tb_gather_init(), "gather init"))
+      chk(tb_gather_init(), "gather init") || chk(tb_reml_init(), "reml kernel init"))
     return bail("");
   *out = c;
   return 0;
@@ -933,6 +967,7 @@ int tb_clone(const tb_ctx* src, int device, tb_ctx** out) {
   c->storage = src->storage;
   c->n_sm = prop.multiProcessorCount;
   c->y_univ = src->y_univ;
+  c->has_pheno = src->has_pheno;
   c->pos_of = src->pos_of;
   if (cudaSetDevice(device) != cudaSuccess) return bail("cudaSetDevice failed");
   auto chk = [&](cudaError_t ce, const char* what) {
@@ -965,7 +1000,8 @@ int tb_clone(const tb_ctx* src, int device, tb_ctx** out) {
   if (chk(cudaStreamSynchronize(c->stream), "peer copy")) return bail("");
   if (chk(tb_gram_tc_init(), "gram kernel init") || chk(tb_chol_init(), "cholesky kernel init") ||
       chk(tb_solve_init(), "solve kernel init") || chk(tb_chol_tc_init(), "tensor-core cholesky init") ||
-      chk(tb_solve_mixed_init(), "mixed solve init") || chk(tb_gather_init(), "gather init"))
+      chk(tb_solve_mixed_init(), "mixed solve init") || chk(tb_gather_init(), "gather init") ||
+      chk(tb_reml_init(), "reml kernel init"))
     return bail("");
   *out = c;
   return 0;
@@ -995,6 +1031,7 @@ int tb_set_rowset(tb_ctx* c, int slot, const int32_t* train, int n_t, const int3
   if (!c) return -1;
   if (slot < 0 || slot >= TB_MAX_SLOTS) return fail(c, "tb_set_rowset: slot out of range");
   if (!train || !valid || n_t < 2 || n_v < 2) return fail(c, "tb_set_rowset: need at least 2 training and 2 validation animals");
+  if (!c->has_pheno) return fail(c, "tb_set_rowset: this context was created without phenotypes");
   TB_CUDA(c, cudaSetDevice(c->device));
   TB_CUDA(c, cudaStreamSynchronize(c->stream));
   TbRowSet& r = c->slots[slot];

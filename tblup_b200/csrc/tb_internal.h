@@ -76,7 +76,8 @@ struct TbCtx {
   int storage = 0;
   TbGeno geno() const { return TbGeno{d_x, ldn, d_x2, ldn / 4}; }
   int* d_colsum_all = nullptr;    // [m]
-  std::vector<double> y_univ;     // phenotypes in universe order
+  std::vector<double> y_univ;     // phenotypes in universe order (zeros when has_pheno is false)
+  bool has_pheno = true;          // false: created without phenotypes (y = NULL), it only scores animals
   std::vector<int> pos_of;        // original animal index -> universe position
   TbRowSet slots[TB_MAX_SLOTS];
   cudaStream_t stream = nullptr;
@@ -321,6 +322,31 @@ cudaError_t tb_chol_tc_factor(float* L32, float* Linv32, void* L16, float* Linv2
                               void (*mark)(void*, int, int), void* mark_ctx, const TbFromC* from_c = nullptr,
                               int t16 = 1, int epi_warps = 16, int chain_fused_jobs = 0, int panel_fused = 1);
 
+// reml.cu: restricted log-likelihood of one (genome, h2) job after the fp64 factorisation of A = G_TT + lambda I
+struct TbRemlJob {
+  const double* M;       // [ntp][ntp] L (lower triangle) as chol.cu leaves it
+  const double* Linv;    // [ntp / TB_NB][TB_NB][TB_NB] inverses of its diagonal blocks
+  const double* y;       // [ntp] training phenotypes minus their mean (zero padded)
+  const int* status;     // non-zero: a pivot was not positive
+  double ymean;          // mean training phenotype (mu = ymean + b / a)
+  int n_t, ntp;
+  double* loglik;        // one value each
+  double* sigma_g2;
+  double* mu;
+};
+cudaError_t tb_reml_init();
+cudaError_t tb_launch_reml(const TbRemlJob* d_jobs, int n_jobs, int max_ntp, cudaStream_t st);
+// one chunk of a REML profile for eval_core: jobs (staged genome g, point s) for s < n, h2 of the job
+// h2[g * ld + s0 + s] (ld = 0: one list shared by every genome), outputs at [g][n_out] entry s0 + s (device)
+struct TbRemlReq {
+  const double* h2;
+  long long ld;
+  int s0, n, n_out;
+  double* d_loglik;
+  double* d_sigma_g2;
+  double* d_mu;
+};
+
 // microbench.cu
 cudaError_t tb_microbench_dmma(int n_sm, cudaStream_t st, double* tflops);
 cudaError_t tb_microbench_umma(int which, int n_sm, cudaStream_t st, double* tops);
@@ -331,5 +357,8 @@ int tb_internal_eval_device(TbCtx* c, const int32_t* slots, int n_slots, double 
 // the same on ONE row set, also writing every genome's solution: d_alpha [P][ntp of the row set], entry i of genome g
 // belonging to the training animal at d_tpos[i] of the row set (entries beyond n_t are padding) -- used by tb_fit_effects
 int tb_internal_eval_alpha(TbCtx* c, int slot, double h2, int mode_rule, double* d_fit, double* d_alpha);
+// REML jobs (genome x h2 point) on ONE row set: gather, centring terms and Gram once per genome, then one fp64 A =
+// G_TT + lambda_job I per job (no G_vt rows), the fp64 Cholesky whatever `precision` says, and reml_kernel
+int tb_internal_eval_reml(TbCtx* c, int slot, int mode_rule, const TbRemlReq* req);
 void tb_internal_collect_spans(TbCtx* c);
 void tb_de_release(TbCtx* c);

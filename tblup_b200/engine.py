@@ -94,11 +94,11 @@ class GblupEngine:
             g, layout = as_dosage_int8(geno), LAYOUT_INT8_ANIMAL_MAJOR
             shape = g.shape
         self.has_phenotypes = pheno is not None
-        if pheno is None:
-            pheno = np.zeros(shape[0])
-        y = np.ascontiguousarray(np.asarray(pheno, dtype=np.float64).ravel())
-        if y.shape[0] != shape[0]:
-            raise ValueError("phenotype vector has %d entries for %d animals" % (y.shape[0], shape[0]))
+        y = None
+        if pheno is not None:
+            y = np.ascontiguousarray(np.asarray(pheno, dtype=np.float64).ravel())
+            if y.shape[0] != shape[0]:
+                raise ValueError("phenotype vector has %d entries for %d animals" % (y.shape[0], shape[0]))
         self.n, self.m = shape
         self.storage = storage
         p = None
@@ -106,7 +106,8 @@ class GblupEngine:
             p = np.ascontiguousarray(np.asarray(perm, dtype=np.int32))
             if p.shape != (self.n,):
                 raise ValueError("perm must list every animal exactly once")
-        rc = self._lib.tb_create_ex(g.ctypes.data, layout, STORAGE[storage], self.n, self.m, y.ctypes.data,
+        rc = self._lib.tb_create_ex(g.ctypes.data, layout, STORAGE[storage], self.n, self.m,
+                                    y.ctypes.data if y is not None else None,
                                     p.ctypes.data if p is not None else None, int(device), C.byref(self._ctx))
         if rc != 0:
             self._ctx = C.c_void_p()
@@ -239,6 +240,36 @@ class GblupEngine:
                                                  centre.ctypes.data, effects.ctypes.data, intercept.ctypes.data,
                                                  a.ctypes.data, a.size, out.ctypes.data), "tb_predict_effects")
         return out
+
+    # -- REML heritability --------------------------------------------------------------------------
+    def reml_profile(self, genomes, h2, slot=0, mode=MODE_AUTO):
+        """Restricted log-likelihood of each genome's model on row set ``slot`` at heritabilities ``h2``: one list
+        (G,) shared by every genome, or (P, G), one list per genome.  Returns arrays (P, G) of l, sigma_g^2 and mu
+        (include/tblup_b200.h, tb_reml_profile, states the model).  Always fp64, whatever ``set_precision`` says; a
+        point whose factorisation fails is NaN.  The genomes become the staged batch (``stage``)."""
+        flat, off = pack_genomes(genomes, self.m)
+        P = off.size - 1
+        h = np.ascontiguousarray(np.asarray(h2, dtype=np.float64))
+        if h.ndim == 1:
+            per_genome = 0
+        elif h.ndim == 2 and h.shape[0] == P:
+            per_genome = 1
+        else:
+            raise ValueError("h2 must be one list of values or one list per genome, got shape %r for %d genomes"
+                             % (h.shape, P))
+        G = h.shape[-1]
+        self.stage(flat=flat, off=off)
+        out = np.empty((3, P, G), dtype=np.float64)
+        self._check(self._lib.tb_reml_profile(self._ctx, int(slot), int(mode), h.ctypes.data, G, per_genome,
+                                              out[0].ctypes.data, out[1].ctypes.data, out[2].ctypes.data),
+                    "tb_reml_profile")
+        return out[0], out[1], out[2]
+
+    def estimate_h2(self, genomes, slot=0, mode=MODE_AUTO, tol=1e-4, bounds=(0.01, 0.99)):
+        """REML estimate of h2 for each genome on row set ``slot``: a list of ``reml.H2Estimate`` (the search is
+        described in ``tblup_b200.reml``)."""
+        from .reml import estimate_h2
+        return estimate_h2(self, genomes, slot=slot, mode=mode, tol=tol, bounds=bounds)
 
     # -- per-marker statistics (top-SNPs seeder, tblup/seeder.py:144-160) ------------------------
     def marker_stats(self, animals, weights):

@@ -326,6 +326,16 @@ class BlupParallelEvaluator(ParallelEvaluator):
             animals = self.testing_indices
         return self.consumers[0].predict([model], animals)[0]
 
+    # ---- REML heritability ------------------------------------------------------------------------------------
+    def estimate_h2(self, genome=None, **search):
+        """REML estimate (``reml.H2Estimate``) of h2 on the training animals (row set 0) for ``genome``, by default
+        every marker: the ``h2`` to run this evaluator with.  On the first engine, like ``fit_model``; ``search``
+        passes ``tol`` / ``bounds`` on to ``GblupEngine.estimate_h2``."""
+        if len(self.consumers) == 0:
+            raise AttributeError("Workers are not set up.")
+        g = np.arange(self.n_columns) if genome is None else np.asarray(genome).astype(int)
+        return self.consumers[0].estimate_h2([g], slot=0, mode=MODE_AUTO, **search)[0]
+
 
 class InterGCVBlupParallelEvaluator(BlupParallelEvaluator):
     """Validation fold rotates with the generation (evaluator.py:434-491)."""
