@@ -44,7 +44,8 @@ enum {
   TB_DBG_PRED = 5,  /* double [n_v]                                                                  */
   TB_DBG_DIMS = 6,  /* int32  [4]              rpad, ntp, n_v, kstride                               */
   TB_DBG_L32 = 7,   /* float  [ntp*ntp]        TF32 Cholesky factor (mixed precision mode only)      */
-  TB_DBG_SWEEPS = 8 /* int32  [1]              refinement sweeps the solve needed (mixed mode)       */
+  TB_DBG_SWEEPS = 8, /* int32 [1]              refinement sweeps the solve needed (mixed mode)       */
+  TB_DBG_LINV32 = 9  /* float [ntp/64][64][64]  inverses of the 64x64 diagonal blocks the solve applies (mixed mode) */
 };
 
 int tb_abi_version(void);

@@ -391,6 +391,7 @@ int eval_core(TbCtx* c, const int32_t* slots, int n_slots, double h2, int mode_r
     if (reml) h_reml.resize(n_jobs);
     c->dbg.L32 = d_L32;
     c->dbg.L16 = d_L16;
+    c->dbg.Linv32 = d_Linv32;
     c->dbg.sweeps = d_sweeps;
     c->dbg.ntp_all = max_ntp;
     c->dbg.W = Wc;
@@ -1388,6 +1389,9 @@ int tb_debug_fetch(tb_ctx* c, int what, int job, void* out, size_t nbytes) {
       if (!d.L32) return fail(c, "tb_debug_fetch: no fp32 factor (fp64 precision mode)");
       src = d.L32 + (size_t)job * d.ntp_all * d.ntp_all; need = (size_t)d.ntp_all * d.ntp_all * 4; break;
     case 8: src = d.sweeps + job; need = 4; break;
+    case TB_DBG_LINV32:
+      if (!d.Linv32) return fail(c, "tb_debug_fetch: no diagonal-block inverses (fp64 precision mode)");
+      src = d.Linv32 + (size_t)job * d.ntp_all * TB_NB; need = (size_t)d.ntp_all * TB_NB * 4; break;
     case TB_DBG_M:
       if (!d.M[job]) return fail(c, "tb_debug_fetch: [A ; G_vt] is not formed in mixed precision mode");
       src = d.M[job]; need = (size_t)(d.ntp[job] + d.n_v[job]) * d.ntp[job] * 8; break;

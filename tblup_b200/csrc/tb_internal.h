@@ -144,7 +144,8 @@ struct TbCtx {
     int W = 0, n_slots = 0, rpad = 0, kstride = 0, centre_shared = 0;
     int32_t* C = nullptr; long long* s = nullptr; long long* SQ = nullptr;
     std::vector<double*> M, alpha, pred;
-    float* L32 = nullptr; const unsigned short* L16 = nullptr; int* sweeps = nullptr; int ntp_all = 0;
+    float* L32 = nullptr; const unsigned short* L16 = nullptr; const float* Linv32 = nullptr; int* sweeps = nullptr;
+    int ntp_all = 0;
     std::vector<int> ntp, n_v;
   } dbg;
   // on-device differential evolution (de.cu)

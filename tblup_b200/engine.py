@@ -14,7 +14,7 @@ from . import _lib
 
 MODE_AUTO, MODE_GBLUP, MODE_SNPBLUP = 0, 1, 2
 STAGES = ["h2d", "gather", "centre", "gram", "scale", "chol_update", "chol_panel", "solve", "d2h"]
-DBG_C, DBG_S, DBG_SQ, DBG_M, DBG_ALPHA, DBG_PRED, DBG_DIMS, DBG_L32, DBG_SWEEPS = range(9)
+DBG_C, DBG_S, DBG_SQ, DBG_M, DBG_ALPHA, DBG_PRED, DBG_DIMS, DBG_L32, DBG_SWEEPS, DBG_LINV32 = range(10)
 PRECISION_MIXED, PRECISION_FP64 = 0, 1
 LAYOUT_INT8_ANIMAL_MAJOR, LAYOUT_PACKED2_SNP_MAJOR = 0, 1
 STORAGE = {"int8": 0, "packed2": 1}
@@ -327,6 +327,7 @@ class GblupEngine:
             DBG_PRED: ((d["n_v"],), np.float64),
             DBG_L32: ((d["ntp"], d["ntp"]), np.float32),
             DBG_SWEEPS: ((1,), np.int32),
+            DBG_LINV32: ((d["ntp"] // 64, 64, 64), np.float32),
         }[what]
         out = np.empty(shape, dtype=dt)
         self._check(self._lib.tb_debug_fetch(self._ctx, what, job, out.ctypes.data, out.nbytes), "tb_debug_fetch")
