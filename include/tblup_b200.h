@@ -149,7 +149,12 @@ int tb_set_option(tb_ctx* ctx, const char* name, long long value);
 /* Facts about the last evaluation / the context: "last_c16", "last_fused_scale", "last_mixed", "last_wave",
  * "storage", "wide_panel", "panel_fused", "de_removed" (size of the removed-marker set), "staged" (genomes staged), "last_fp4", "last_perm", "last_split",
  * "last_fallbacks" (jobs of the last evaluation whose mixed-precision solve gave up -- pivot breakdown or no
- * convergence, h2 close to 1 -- and that were evaluated again with the fp64 Cholesky). */
+ * convergence, h2 close to 1 -- and that were evaluated again with the fp64 Cholesky),
+ * "last_solve" (the instantiation of the mixed-precision solve the last wave launched, as bits: TB_SOLVE_CONTIG
+ * training animals at consecutive positions, TB_SOLVE_BIG alpha in global memory (more than 4 096 padded training
+ * animals), TB_SOLVE_C16 int16 cross-products, TB_SOLVE_HOLE prefix-with-one-aligned-hole kernels, TB_SOLVE_PAIR two
+ * CTAs per matrix; -1 when the last evaluation ran no mixed-precision solve). */
+enum { TB_SOLVE_CONTIG = 1, TB_SOLVE_BIG = 2, TB_SOLVE_C16 = 4, TB_SOLVE_HOLE = 8, TB_SOLVE_PAIR = 16 };
 int tb_get_info(const tb_ctx* ctx, const char* name, long long* value);
 /* Offsets (P + 1 entries, P = tb_get_info "staged") of the ragged batch currently staged on the device. */
 int tb_staged_offsets(const tb_ctx* ctx, int64_t* off_out, int n);

@@ -261,6 +261,7 @@ int eval_core(TbCtx* c, const int32_t* slots, int n_slots, double h2, int mode_r
   bool mixed = !reml && c->precision == 0 && tb_solve_mixed_fits(max_ntp) && 4LL * kmax < (1LL << 23);
   for (int s = 0; s < n_slots; ++s) mixed = mixed && sv[s].rs->ntp == max_ntp;
   c->last_mixed = mixed ? 1 : 0;
+  c->last_solve = -1;
   if (allow_fallback) c->last_fallbacks = 0;
   if (mixed) {
     const size_t need = (size_t)P * n_slots;
@@ -593,7 +594,7 @@ int eval_core(TbCtx* c, const int32_t* slots, int n_slots, double h2, int mode_r
         hole = hole || (!use_perm && sv[s].rs->gap > 0);
       }
       TB_CUDA(c, tb_launch_solve_mixed(d_msolve, n_jobs, max_ntp, contig ? 1 : 0, c16 ? 1 : 0, hole ? 1 : 0, st, c->n_sm,
-                                       c->solve_pair));
+                                       c->solve_pair, &c->last_solve));
       span_end(c, sp);
       count(c, TB_ST_SOLVE, 1);
       if (d_alpha)
@@ -690,6 +691,7 @@ int fp64_fallback(TbCtx* c, const int32_t* slots, int n_slots, double h2, int mo
   const size_t keep_cap = c->idx_cap;
   const int keep_P = c->P, keep_prec = c->precision;
   const int keep_c16 = c->last_c16, keep_fused = c->last_fused, keep_fp4 = c->last_fp4, keep_wave = c->last_wave;
+  const int keep_solve = c->last_solve;
   c->h_off = sub_off;
   c->d_idx = d_sub;
   c->idx_cap = (size_t)sub_off.back();
@@ -706,6 +708,7 @@ int fp64_fallback(TbCtx* c, const int32_t* slots, int n_slots, double h2, int mo
   c->last_fused = keep_fused;
   c->last_fp4 = keep_fp4;
   c->last_wave = keep_wave;
+  c->last_solve = keep_solve;
   if (rc == 0) {
     for (size_t j = 0; j < redo.size(); ++j)
       for (int s = 0; s < n_slots; ++s)
@@ -1482,6 +1485,7 @@ int tb_get_info(const tb_ctx* c, const char* name, long long* value) {
   else if (s == "de_removed") *value = c->de.n_banned;
   else if (s == "last_fp4") *value = c->last_fp4;
   else if (s == "last_perm") *value = c->last_perm;
+  else if (s == "last_solve") *value = c->last_solve;
   else if (s == "last_split") *value = c->last_split;
   else if (s == "last_fallbacks") *value = c->last_fallbacks;
   else if (s == "last_issue_us") *value = c->last_issue_us;

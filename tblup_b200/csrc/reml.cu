@@ -201,7 +201,7 @@ extern "C" int tb_reml_profile(tb_ctx* c, int slot, int mode_rule, const double*
   // put back, and workspace grown for the fp64 matrices of the profile (up to 80 % of the free HBM) is released
   const int keep_mixed = c->last_mixed, keep_c16 = c->last_c16, keep_fused = c->last_fused, keep_fp4 = c->last_fp4;
   const int keep_wave = c->last_wave, keep_perm = c->last_perm, keep_split = c->last_split;
-  const int keep_fallbacks = c->last_fallbacks;
+  const int keep_fallbacks = c->last_fallbacks, keep_solve = c->last_solve;
   const long long keep_issue = c->last_issue_us;
   const size_t keep_ws = c->ws_bytes;
   TbRemlReq req{h2, per_genome ? (long long)n_h2 : 0LL, 0, 0, n_h2, d_out, d_out + n_out, d_out + 2 * n_out};
@@ -236,6 +236,7 @@ extern "C" int tb_reml_profile(tb_ctx* c, int slot, int mode_rule, const double*
   c->last_perm = keep_perm;
   c->last_split = keep_split;
   c->last_fallbacks = keep_fallbacks;
+  c->last_solve = keep_solve;
   c->last_issue_us = keep_issue;
   if (rc) return rc;
   if (ce != cudaSuccess) return rfail(c, std::string("tb_reml_profile: D2H: ") + cudaGetErrorString(ce), -2);

@@ -1000,7 +1000,7 @@ bool tb_solve_mixed_fits(int ntp) { return solve_mixed_smem_bytes(ntp) <= 220 * 
 // (vectorised symmetric mat-vec); otherwise positions are looked up per element.
 // hole != 0 (with contiguous and c16): some row set is contiguous with one aligned hole (see TbRowSet).
 cudaError_t tb_launch_solve_mixed(const TbSolveMixedJob* d_jobs, int n_jobs, int ntp, int contiguous, int c16, int hole,
-                                  cudaStream_t st, int n_sm, int pair_mode) {
+                                  cudaStream_t st, int n_sm, int pair_mode, int* variant) {
   const int smem = solve_mixed_smem_bytes(ntp);
   if (smem > g_solve_mixed_smem_max) return cudaErrorInvalidConfiguration;
   const bool big = ntp > MIXED_SMEM_NTP;
@@ -1008,6 +1008,9 @@ cudaError_t tb_launch_solve_mixed(const TbSolveMixedJob* d_jobs, int n_jobs, int
   // 2 always); contiguous kernels only
   const int slots = n_sm * ((smem + 1024) * 2 <= 228 * 1024 ? 2 : 1);
   const bool pair = contiguous && pair_mode != 0 && (pair_mode == 2 || 2 * n_jobs <= slots);
+  // the instantiation launched below, as the TB_SOLVE_* bits of tb_get_info "last_solve"
+  if (variant)
+    *variant = (contiguous ? 1 : 0) | (big ? 2 : 0) | (c16 ? 4 : 0) | (hole && contiguous && c16 ? 8 : 0) | (pair ? 16 : 0);
   if (pair) {
     cudaLaunchConfig_t cfg = {};
     cfg.gridDim = dim3(2 * n_jobs);

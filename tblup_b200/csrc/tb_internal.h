@@ -116,6 +116,7 @@ struct TbCtx {
   int last_fp4 = 0;
   int narrow_c = 1;               // 1: int16 cross-products when every genome of the batch has 4 k <= 32 767
   int last_c16 = 0;
+  int last_solve = -1;            // TB_SOLVE_* bits of the mixed solve the last wave launched, -1: none (fp64 path)
   double* d_fit_out = nullptr;    // device staging of the fitness vector for host-output calls
   size_t fit_cap = 0;
   int* d_fail = nullptr;          // [P * n_slots] per-job "mixed precision gave up" flags of the last evaluation
@@ -293,7 +294,7 @@ cudaError_t tb_solve_mixed_init();
 void tb_solve_mixed_set_debug(int v);
 bool tb_solve_mixed_fits(int ntp);
 cudaError_t tb_launch_solve_mixed(const TbSolveMixedJob* d_jobs, int n_jobs, int ntp, int contiguous, int c16, int hole,
-                                  cudaStream_t st, int n_sm = 148, int pair_mode = 1);
+                                  cudaStream_t st, int n_sm = 148, int pair_mode = 1, int* variant = nullptr);
 // col_end > 0: only columns [0, col_end) (the first outer block column of the factorisation)
 cudaError_t tb_launch_scale32(const TbScaleJob* d_jobs, int n_jobs, int ntp, float* L32, int c16, cudaStream_t st,
                               int col_end = 0);

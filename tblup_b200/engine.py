@@ -16,6 +16,7 @@ MODE_AUTO, MODE_GBLUP, MODE_SNPBLUP = 0, 1, 2
 STAGES = ["h2d", "gather", "centre", "gram", "scale", "chol_update", "chol_panel", "solve", "d2h"]
 DBG_C, DBG_S, DBG_SQ, DBG_M, DBG_ALPHA, DBG_PRED, DBG_DIMS, DBG_L32, DBG_SWEEPS, DBG_LINV32 = range(10)
 PRECISION_MIXED, PRECISION_FP64 = 0, 1
+SOLVE_CONTIG, SOLVE_BIG, SOLVE_C16, SOLVE_HOLE, SOLVE_PAIR = 1, 2, 4, 8, 16      # tb_get_info "last_solve"
 LAYOUT_INT8_ANIMAL_MAJOR, LAYOUT_PACKED2_SNP_MAJOR = 0, 1
 STORAGE = {"int8": 0, "packed2": 1}
 
@@ -363,7 +364,9 @@ class GblupEngine:
         return {0: "mixed", 1: "fp64"}[int(self._lib.tb_last_precision(self._ctx))]
 
     def info(self, name):
-        """Facts about the last evaluation: 'last_c16', 'last_fused_scale', 'last_mixed', 'last_wave', 'storage'."""
+        """Facts about the last evaluation: 'last_c16', 'last_fused_scale', 'last_mixed', 'last_wave', 'storage',
+        'last_solve' (SOLVE_* bits of the mixed-precision solve kernel the last wave ran, -1: none) and the others
+        include/tblup_b200.h lists."""
         v = C.c_longlong(0)
         if self._lib.tb_get_info(self._ctx, name.encode(), C.byref(v)) != 0:
             raise KeyError(name)

@@ -105,7 +105,7 @@ def test_per_genome_points_and_waves(small):
 def test_fitness_is_unchanged_by_a_profile(small, precision):
     genomes = _genomes([500, 1300, 900], seed=8)
     info = ("last_c16", "last_fused_scale", "last_mixed", "last_wave", "last_fp4", "last_perm", "last_split",
-            "last_fallbacks", "storage", "wide_panel", "t16", "panel_fused", "epi_warps")
+            "last_fallbacks", "last_solve", "storage", "wide_panel", "t16", "panel_fused", "epi_warps")
     with _engine(small, "packed2") as eng:
         eng.set_precision(precision)
         before = eng.evaluate(genomes, slots=[0, 2], h2=0.4)
