@@ -192,7 +192,11 @@ int tb_microbench(tb_ctx* ctx, int which, double* out);
  * (evolver.py:147-151), take_out [P] (nullable) receives which children replaced their parent.
  * tb_de_get: what = 0 population fitness [P] f64, 1 last offspring fitness [P] f64, 2 population keys [P][m] f64,
  * 3 last offspring keys, 4 decoded genome of individual `which` [length] i32 (ascending index order),
- * 5 genomes of the last evaluated batch [P][length] i32. */
+ * 5 genomes of the last evaluated batch [P][length] i32, 9 parent picks of the last generation [P][3] i32 (host
+ * abc or device draws), 10 forced crossover positions of the last generation [P] i32.  Items 9 and 10 are read-only
+ * debug items; they fail until a generation has been evolved.
+ * Decode order: the `length` largest keys in numpy's order (-0.0 == +0.0; every NaN equal to every other and above
+ * +inf), ties at the threshold taken lowest index first; the list comes back in ascending index order. */
 int tb_de_init(tb_ctx* ctx, int P, int length, const double* keys_host, uint64_t seed);
 int tb_de_evaluate(tb_ctx* ctx, const int32_t* slots, int n_slots, double h2, int mode_rule);
 int tb_de_step(tb_ctx* ctx, const int32_t* slots, int n_slots, double h2, int mode_rule, double F, double CR, int clip,

@@ -74,12 +74,21 @@ __global__ void __launch_bounds__(256) de_evolve_kernel(const double* __restrict
                  kc = keys[(size_t)abc[3 * i + 2] * m + j];
     v = __dadd_rn(ka, __dmul_rn(F, __dsub_rn(kb, kc)));   // numpy's a + mi * (b - c): three roundings, no fma
   }
-  if (clip) v = fmin(fmax(v, 0.0), (double)(m - 1));
+  // np.clip(v, 0, m - 1): NaN and -0.0 pass through unchanged (fmin / fmax would turn a NaN into a bound)
+  if (clip) {
+    const double hi = (double)(m - 1);
+    v = v < 0.0 ? 0.0 : v;
+    v = v > hi ? hi : v;
+  }
   child[row + j] = v;
 }
 
+// Order-preserving map of a key to an unsigned integer, in numpy's sort order: -0.0 and +0.0 are one value, and every
+// NaN (either sign, any payload) is one value above +inf.  Keys numpy holds equal therefore map to one integer, and
+// the decode's tie rule (lowest index first) covers them all.
 __device__ __forceinline__ unsigned long long sortable(double d) {
-  const unsigned long long b = (unsigned long long)__double_as_longlong(d);
+  unsigned long long b = (unsigned long long)__double_as_longlong(d);
+  b = d != d ? 0x7FF8000000000000ULL : d == 0.0 ? 0ULL : b;
   return (b >> 63) ? ~b : (b | 0x8000000000000000ULL);
 }
 
@@ -524,6 +533,7 @@ int tb_de_step_begin(tb_ctx* c, const int32_t* slots, int n_slots, double h2, in
     TB_CUDA(c, cudaGetLastError());
     c->launches += 1;
   }
+  d.drawn = true;
   const unsigned char* d_mask = nullptr;
   if (mask) {
     if (!d.mask) TB_CUDA(c, cudaMalloc(&d.mask, (size_t)P * m));
@@ -643,14 +653,14 @@ int tb_de_evaluate_testing(tb_ctx* c, int slot, double h2, int mode_rule, double
   if (!fitness_out) return de_fail(c, "tb_de_evaluate_testing: null output");
   TB_CUDA(c, cudaSetDevice(c->device));
   const int stride = d.k + d.n_banned;
+  const size_t smem = ((size_t)(c->m + 31) / 32) * 4;                                 // membership bitmap, m bits
+  if (d.n_banned && smem > 200 * 1024) return de_fail(c, "tb_de_evaluate_testing: marker bitmap exceeds shared memory");
   std::vector<int> h_lens;
   if (int rc = de_ensure_rows(c, stride)) return rc;
   de_decode_kernel<<<d.P, 1024, 0, c->stream>>>(d.keys, c->m, d.k, d.rows, stride);   // room for the removed markers
   TB_CUDA(c, cudaGetLastError());
   c->launches += 1;
   if (d.n_banned) {
-    const size_t smem = ((size_t)(c->m + 31) / 32) * 4;
-    if (smem > 200 * 1024) return de_fail(c, "tb_de_evaluate_testing: marker bitmap exceeds shared memory");
     if (smem > 48 * 1024)
       TB_CUDA(c, cudaFuncSetAttribute(de_union_banned_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     de_union_banned_kernel<<<d.P, 1024, smem, c->stream>>>(d.rows, stride, d.k, c->m, d.banned_list, d.n_banned, d.lens);
@@ -713,6 +723,12 @@ int tb_de_get(tb_ctx* c, int what, int which, void* out, size_t nbytes) {
       if ((int)c->h_off.size() < c->P + 1 || c->P <= 0) return de_fail(c, "tb_de_get: no batch staged");
       src = c->d_idx; need = (size_t)c->h_off[c->P] * 4; break;
     }
+    case 9:                                                                       // parent picks of the last step [P][3]
+      if (!d.drawn) return de_fail(c, "tb_de_get: no generation has been evolved yet");
+      src = d.abc; need = (size_t)d.P * 3 * 4; break;
+    case 10:                                                                      // forced crossover positions [P]
+      if (!d.drawn) return de_fail(c, "tb_de_get: no generation has been evolved yet");
+      src = d.fixed; need = (size_t)d.P * 4; break;
     default: return de_fail(c, "tb_de_get: unknown item");
   }
   if (nbytes < need) return de_fail(c, "tb_de_get: buffer too small");

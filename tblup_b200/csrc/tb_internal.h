@@ -155,6 +155,7 @@ struct TbCtx {
     double *keys = nullptr, *child = nullptr, *fit = nullptr, *child_fit = nullptr, *raw_fit = nullptr;
     size_t raw_cap = 0;
     int *abc = nullptr, *fixed = nullptr, *take = nullptr;
+    bool drawn = false;                  // abc / fixed hold the draws of a generation (tb_de_get 9, 10)
     unsigned char* mask = nullptr;
     // SNP removal (tblup/evaluator.py:589-633): flags per marker, the same set as an ascending list, scratch rows
     unsigned char* banned = nullptr;

@@ -187,6 +187,10 @@ class DeviceDE:
         """Decoded genome of individual ``i`` (the set of its ``length`` largest keys, ascending marker index)."""
         return self._get(4, (self.k,), np.int32, which=i)
 
+    def last_draws(self):
+        """(abc [P, 3], fixed [P]) of the last generation: the host's draws, or the ones made on the device."""
+        return self._get(9, (self.P, 3), np.int32), self._get(10, (self.P,), np.int32)
+
     def last_genomes(self):
         """Genomes of the last scored batch, (staged, k); only meaningful while no marker is removed (fixed length)."""
         return self._get(5, (self._staged(), self.k), np.int32)

@@ -64,28 +64,48 @@ def test_device_de_replays_reference_generations(name):
         eng.close()
 
 
+DECODE_M = [257, 1023, 1024, 1025, 4097, 50_000, 500_000]
+
+
+def _decode_engine(m):
+    from tblup_b200 import GblupEngine, synth
+    x, y = synth.synth_dataset(64, m, h2=0.4, seed=m)
+    tr, va, te = synth.split_indices(64, seed=m)
+    eng = GblupEngine(x, y, perm=np.concatenate([tr, va, te]))
+    eng.set_rowset(0, tr, va)
+    return eng
+
+
 def test_decode_matches_argsort_top_k_with_ties_and_negatives():
+    """Both device decodes -- one CTA per call (``genome``) and the batched decode behind ``evaluate`` (``last_genomes``,
+    ``last_lists``) -- against ``D.decode_ordered`` as exact index arrays: numpy's order (-0.0 == +0.0, every NaN equal
+    and above +inf), ties at the threshold taken lowest index first.  m runs from one chunk (257) across the 1 024-key
+    chunk edges to 500 000 markers, the length from 1 to m.  The key families (oracle/de_oracle.py) put the threshold
+    on ties spread over several chunks, on +-0, NaN of both signs, +-inf, keys equal in their top 7 bytes, subnormals
+    and magnitudes near DBL_MAX; with distinct keys the result is numpy's own top-k."""
     from tblup_b200.de import DeviceDE
-    eng, *_ = _engine(257)
-    try:
-        rng = np.random.default_rng(0)
-        keys = rng.normal(size=(6, 257))
-        keys[1, :50] = 0.25                      # a block of ties straddling the threshold
-        keys[2] = np.round(keys[2], 1)           # many ties
-        keys[3] = -np.abs(keys[3])               # all negative
-        keys[4, ::3] = -0.0
-        for length in (1, 40, 256, 257):
-            de = DeviceDE(eng, 6, length, keys=keys)
-            for i in range(6):
-                got = de.genome(i)
-                assert len(np.unique(got)) == length and np.all(np.diff(got) > 0)
-                thr = np.sort(keys[i])[257 - length]
-                assert np.all(keys[i][got] >= thr)                               # nothing below the k-th largest key
-                assert np.all(keys[i][np.setdiff1d(np.arange(257), got)] <= thr)
-                if len(np.unique(keys[i])) == 257:
-                    assert np.array_equal(got, np.sort(D.decode(keys[i], length)))
-    finally:
-        eng.close()
+    for m in DECODE_M:
+        eng = _decode_engine(m)
+        try:
+            lengths = sorted({1, 2, 40, 1023, 1024, 1025, 5001, m - 1, m} & set(range(1, m + 1)))
+            for length in lengths:
+                fam = D.decode_key_families(m, length, seed=length)
+                names = list(fam)
+                keys = np.stack([fam[nm] for nm in names])
+                de = DeviceDE(eng, len(names), length, keys=keys)
+                want = [D.decode_ordered(kv, length) for kv in keys]
+                for i, nm in enumerate(names):
+                    got = de.genome(i)
+                    assert np.array_equal(got, want[i]), (m, length, nm)
+                    if np.unique(keys[i]).size == m:
+                        assert np.array_equal(got, np.sort(D.decode(keys[i], length)))
+                de.evaluate(slots=[0], h2=0.4)
+                batch, lists = de.last_genomes(), de.last_lists()
+                for i, nm in enumerate(names):
+                    assert np.array_equal(batch[i], want[i]) and np.array_equal(lists[i], want[i]), (m, length, nm)
+            print("DE_SCALE decode m=%d: lengths %s x %d key families exact" % (m, lengths, len(names)), flush=True)
+        finally:
+            eng.close()
 
 
 def test_device_driven_generations_improve_fitness():
