@@ -150,6 +150,41 @@ def exact_gram(x_int, indices, rows):
     return out
 
 
+def gram_blas(x_int, indices, rows, cols=None, chunk=4096):
+    """C[a, b] = sum_j x[rows[a], idx_j] * x[cols[b], idx_j] as int64 (``cols`` None: ``rows``): float64 BLAS products
+    of the gathered dosages, summed over chunks of ``chunk`` markers so that production panels (k = 50 000) need no
+    full gather.  Exact: every partial sum is an integer of at most 4 k, far below 2**53."""
+    x_int = np.asarray(x_int)
+    idx = np.asarray(indices).ravel()
+    rows = np.asarray(rows)
+    cols = rows if cols is None else np.asarray(cols)
+    acc = np.zeros((rows.size, cols.size), dtype=np.float64)
+    for j0 in range(0, idx.size, chunk):
+        cj = idx[j0:j0 + chunk]
+        a = x_int[np.ix_(rows, cj)].astype(np.float64)
+        b = a if cols is rows else x_int[np.ix_(cols, cj)].astype(np.float64)
+        acc += a @ b.T
+    out = np.rint(acc).astype(np.int64)
+    assert np.all(out == acc)
+    return out
+
+
+def row_dots_blas(x_int, indices, rows, weights, chunk=4096):
+    """s[a] = sum_j x[rows[a], idx_j] * weights[j] as int64 for integer weights, chunked like ``gram_blas`` (exact while
+    2 k max|weights| < 2**53); with ``weights`` = the column sums of the frequency animals these are the s_a of
+    ``exact_centring_terms``."""
+    x_int = np.asarray(x_int)
+    idx = np.asarray(indices).ravel()
+    w = np.asarray(weights, dtype=np.int64).ravel()
+    rows = np.asarray(rows)
+    acc = np.zeros(rows.size, dtype=np.float64)
+    for j0 in range(0, idx.size, chunk):
+        acc += x_int[np.ix_(rows, idx[j0:j0 + chunk])].astype(np.float64) @ w[j0:j0 + chunk].astype(np.float64)
+    out = np.rint(acc).astype(np.int64)
+    assert np.all(out == acc)
+    return out
+
+
 def exact_centring_terms(x_int, indices, rows, freq_rows):
     """Integer ingredients of the rank-1 centring.
 

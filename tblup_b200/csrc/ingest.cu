@@ -10,19 +10,23 @@
 namespace {
 
 // rows: [n_rows][m] (m contiguous).  x: [m][ldn], writes x[j][pos0 + r].
+// Row tiles stride by gridDim.y: a chunk of more than 65 535 x 64 animals (few markers) needs no second launch.
 __global__ void transpose_rows_kernel(const int8_t* __restrict__ rows, int n_rows, int m, int8_t* __restrict__ x,
                                       int ldn, int pos0) {
   __shared__ int8_t tile[64][65];
-  const int j0 = blockIdx.x * 64, r0 = blockIdx.y * 64;
+  const int j0 = blockIdx.x * 64;
   const int tx = threadIdx.x, ty = threadIdx.y;  // 64 x 4
-  for (int rr = ty; rr < 64; rr += 4) {
-    int r = r0 + rr, j = j0 + tx;
-    tile[rr][tx] = (r < n_rows && j < m) ? rows[(size_t)r * m + j] : (int8_t)0;
-  }
-  __syncthreads();
-  for (int jj = ty; jj < 64; jj += 4) {
-    int j = j0 + jj, r = r0 + tx;
-    if (j < m && r < n_rows) x[(size_t)j * ldn + pos0 + r] = tile[tx][jj];
+  for (int r0 = blockIdx.y * 64; r0 < n_rows; r0 += gridDim.y * 64) {
+    for (int rr = ty; rr < 64; rr += 4) {
+      int r = r0 + rr, j = j0 + tx;
+      tile[rr][tx] = (r < n_rows && j < m) ? rows[(size_t)r * m + j] : (int8_t)0;
+    }
+    __syncthreads();
+    for (int jj = ty; jj < 64; jj += 4) {
+      int j = j0 + jj, r = r0 + tx;
+      if (j < m && r < n_rows) x[(size_t)j * ldn + pos0 + r] = tile[tx][jj];
+    }
+    __syncthreads();
   }
 }
 
@@ -49,18 +53,20 @@ __global__ void pack2_kernel(const int8_t* __restrict__ x, size_t n_words, uint8
 }
 
 // rows2: [n_rows][stride] packed markers of a chunk, animals in FILE order; x[j0 + r][p] = code of animal perm[p].
-// Code 3 is not a dosage: counted in *bad (the caller rejects the data set).
+// Code 3 is not a dosage: counted in *bad (the caller rejects the data set).  Markers stride by gridDim.y: a chunk is
+// up to 256 MiB of rows, which for fewer than ~16 400 animals is more markers than gridDim.y can hold.
 __global__ void unpack2_perm_kernel(const uint8_t* __restrict__ rows2, int n_rows, int stride, const int* __restrict__ perm,
                                     int n, int8_t* __restrict__ x, int ldn, int j0, int* __restrict__ bad) {
-  const int r = blockIdx.y;
-  const uint8_t* src = rows2 + (size_t)r * stride;
-  int8_t* dst = x + (size_t)(j0 + r) * ldn;
   int local_bad = 0;
-  for (int p = blockIdx.x * blockDim.x + threadIdx.x; p < n; p += gridDim.x * blockDim.x) {
-    const int a = perm[p];
-    const int code = (src[a >> 2] >> (2 * (a & 3))) & 3;
-    local_bad |= code == 3;
-    dst[p] = (int8_t)code;
+  for (int r = blockIdx.y; r < n_rows; r += gridDim.y) {
+    const uint8_t* src = rows2 + (size_t)r * stride;
+    int8_t* dst = x + (size_t)(j0 + r) * ldn;
+    for (int p = blockIdx.x * blockDim.x + threadIdx.x; p < n; p += gridDim.x * blockDim.x) {
+      const int a = perm[p];
+      const int code = (src[a >> 2] >> (2 * (a & 3))) & 3;
+      local_bad |= code == 3;
+      dst[p] = (int8_t)code;
+    }
   }
   if (local_bad) atomicAdd(bad, 1);
 }
@@ -130,14 +136,14 @@ cudaError_t tb_launch_pack2(const int8_t* d_x, int ldn, int m, uint8_t* d_x2, cu
 
 cudaError_t tb_launch_unpack2_perm(const uint8_t* d_rows2, int n_rows, int stride, const int* d_perm, int n,
                                    int8_t* d_x, int ldn, int j0, int* d_bad, cudaStream_t st) {
-  dim3 grid((n + 1023) / 1024 > 8 ? 8 : (n + 1023) / 1024, n_rows);
+  dim3 grid((n + 1023) / 1024 > 8 ? 8 : (n + 1023) / 1024, std::min(n_rows, 65535));
   unpack2_perm_kernel<<<grid, 256, 0, st>>>(d_rows2, n_rows, stride, d_perm, n, d_x, ldn, j0, d_bad);
   return cudaGetLastError();
 }
 
 cudaError_t tb_launch_transpose_rows(const int8_t* d_rows, int n_rows, int m, int8_t* d_x, int ldn, int pos0,
                                      cudaStream_t st) {
-  dim3 grid((m + 63) / 64, (n_rows + 63) / 64), block(64, 4);
+  dim3 grid((m + 63) / 64, std::min((n_rows + 63) / 64, 65535)), block(64, 4);
   transpose_rows_kernel<<<grid, block, 0, st>>>(d_rows, n_rows, m, d_x, ldn, pos0);
   return cudaGetLastError();
 }
