@@ -245,7 +245,8 @@ int tb_marker_stats(tb_ctx* ctx, const int32_t* animals, int n_animals, const do
  * keep_out [k] receives 1 for markers that stay and 0 for knocked-out ones (the reference's `mask`),
  * best_fitness_out the final fitness; n_evals_out (nullable) the evaluations the greedy sequence consumed (= what the
  * reference would have run), n_batches_out (nullable) the batched pipeline passes it took.
- * tb_knockout_scan: fitness_out[i] = blup(genome without its i-th entry) for every i (no greedy dependence). */
+ * tb_knockout_scan: fitness_out[i] = blup(genome without its i-th entry) for every i (no greedy dependence).
+ * Both score their candidates in an index buffer of their own: the staged batch stays staged, errors included. */
 int tb_knockout(tb_ctx* ctx, const int32_t* genome, int k, int slot, double h2, int mode_rule, double start_fitness,
                 uint8_t* keep_out, double* best_fitness_out, int32_t* n_evals_out, int32_t* n_batches_out);
 int tb_knockout_scan(tb_ctx* ctx, const int32_t* genome, int k, int slot, double h2, int mode_rule, double* fitness_out);

@@ -9,10 +9,15 @@
 //   scan in order: the first candidate that improves is accepted (exactly the reference's `fitness > best_fitness`,
 //   NaN never wins); candidates after it were scored with that marker still present, so the next batch starts there.
 //
-// The decisions are therefore the reference's, one for one; a batch costs about what ONE single-genome evaluation
-// costs (the pipeline is latency-bound below ~150 genomes), so the search is between 1x and Bx faster than the
-// sequential loop depending on how often a drop is accepted.  The batch size adapts to the observed acceptance gaps.
+// Each decision compares the fitness of the list the sequential loop would score at that step; a batch costs about what
+// ONE single-genome evaluation costs (the pipeline is latency-bound below ~150 genomes), so the search is between 1x
+// and Bx faster than the sequential loop depending on how often a drop is accepted.  The batch size adapts to the
+// observed acceptance gaps.  A candidate's fitness is the same bits whatever batch it is scored in as long as the
+// mixed-precision solve runs one CTA per matrix (option solve_pair 0; DESIGN section 4 states what the tests hold).
 // tb_knockout_scan is the non-greedy companion: the fitness of every leave-one-out list of a fixed genome.
+//
+// Both calls score their candidates in an index buffer of their own and leave the staged batch (tb_stage_genomes)
+// as they found it, on every way out, errors included: tb_eval_staged afterwards evaluates what the caller staged.
 #include "tb_internal.h"
 #include "../../include/tblup_b200.h"
 
@@ -36,36 +41,47 @@ __global__ void knockout_drop_kernel(const int* __restrict__ src, int L, int q, 
   for (int t = blockIdx.x * blockDim.x + threadIdx.x; t < L - 1; t += gridDim.x * blockDim.x) dst[t] = src[t < q ? t : t + 1];
 }
 
-int ensure_idx(TbCtx* c, size_t total) {
-  if (total > c->idx_cap) {
-    TB_CUDA(c, cudaStreamSynchronize(c->stream));
-    cudaFree(c->d_idx);
-    c->d_idx = nullptr;
-    c->idx_cap = 0;
-    TB_CUDA(c, cudaMalloc(&c->d_idx, total * sizeof(int)));
-    c->idx_cap = total;
-  }
-  return 0;
-}
-
 struct Scratch {
   int* base[2] = {nullptr, nullptr};
   double* fit = nullptr;
+  int* idx = nullptr;             // the candidate lists of one batch
+  size_t idx_cap = 0;
   ~Scratch() {
     cudaFree(base[0]);
     cudaFree(base[1]);
     cudaFree(fit);
+    cudaFree(idx);
   }
 };
 
-// score candidates q0 .. q0 + B - 1 of the base list (length L) on row set `slot` -> h_fit[0 .. B)
-int score_batch(TbCtx* c, const int* d_base, int L, int q0, int B, int slot, double h2, int mode_rule, double* d_fit,
-                std::vector<double>& h_fit) {
-  if (int rc = ensure_idx(c, (size_t)B * (L - 1))) return rc;
+// The caller's staged batch, set aside for the length of one call (the fp64 fallback of api.cu swaps its sub-batch in
+// the same way).  Declared after the Scratch it points into, so that it is put back before that Scratch is freed.
+struct StagedBatch {
+  TbCtx* c;
+  std::vector<long long> off;
+  int* idx;
+  size_t cap;
+  int P;
+  explicit StagedBatch(TbCtx* ctx) : c(ctx), idx(ctx->d_idx), cap(ctx->idx_cap), P(ctx->P) { off.swap(c->h_off); }
+  ~StagedBatch() {
+    c->h_off.swap(off);
+    c->d_idx = idx;
+    c->idx_cap = cap;
+    c->P = P;
+  }
+};
+
+// score candidates q0 .. q0 + B - 1 of the base list (length L) on row set `slot` -> h_fit[0 .. B); the candidate
+// lists go to sc.idx (B (L - 1) entries, allocated by the caller) and are staged from there
+int score_batch(TbCtx* c, Scratch& sc, const int* d_base, int L, int q0, int B, int slot, double h2, int mode_rule,
+                double* d_fit, std::vector<double>& h_fit) {
+  if ((size_t)B * (L - 1) > sc.idx_cap) return ko_fail(c, "internal: knockout batch exceeds its index buffer");
   dim3 grid((unsigned)std::min(32, (L - 1 + 255) / 256), (unsigned)B);
-  knockout_lists_kernel<<<grid, 256, 0, c->stream>>>(d_base, L, q0, c->d_idx);
+  knockout_lists_kernel<<<grid, 256, 0, c->stream>>>(d_base, L, q0, sc.idx);
   TB_CUDA(c, cudaGetLastError());
   c->launches += 1;
+  c->d_idx = sc.idx;
+  c->idx_cap = sc.idx_cap;
   c->h_off.resize(B + 1);
   for (int i = 0; i <= B; ++i) c->h_off[i] = (long long)i * (L - 1);
   c->P = B;
@@ -98,13 +114,16 @@ int tb_knockout_scan(tb_ctx* c, const int32_t* genome, int k, int slot, double h
   if (int rc = check_args(c, genome, k, slot, h2, mode_rule, "tb_knockout_scan")) return rc;
   TB_CUDA(c, cudaSetDevice(c->device));
   Scratch sc;
+  StagedBatch staged(c);
+  sc.idx_cap = (size_t)std::min(k, 1024) * (k - 1);
+  TB_CUDA(c, cudaMalloc(&sc.idx, sc.idx_cap * sizeof(int)));
   TB_CUDA(c, cudaMalloc(&sc.base[0], (size_t)k * sizeof(int)));
   TB_CUDA(c, cudaMalloc(&sc.fit, (size_t)std::min(k, 1024) * sizeof(double)));
   TB_CUDA(c, cudaMemcpyAsync(sc.base[0], genome, (size_t)k * sizeof(int), cudaMemcpyHostToDevice, c->stream));
   std::vector<double> h;
   for (int q0 = 0; q0 < k; q0 += 1024) {
     const int B = std::min(1024, k - q0);
-    if (int rc = score_batch(c, sc.base[0], k, q0, B, slot, h2, mode_rule, sc.fit, h)) return rc;
+    if (int rc = score_batch(c, sc, sc.base[0], k, q0, B, slot, h2, mode_rule, sc.fit, h)) return rc;
     for (int i = 0; i < B; ++i) fitness_out[q0 + i] = h[i];
   }
   return 0;
@@ -117,6 +136,9 @@ int tb_knockout(tb_ctx* c, const int32_t* genome, int k, int slot, double h2, in
   if (int rc = check_args(c, genome, k, slot, h2, mode_rule, "tb_knockout")) return rc;
   TB_CUDA(c, cudaSetDevice(c->device));
   Scratch sc;
+  StagedBatch staged(c);
+  sc.idx_cap = (size_t)std::min(k, 1024) * (k - 1);     // the largest batch: min(k, 1 024) lists of k - 1 markers
+  TB_CUDA(c, cudaMalloc(&sc.idx, sc.idx_cap * sizeof(int)));
   TB_CUDA(c, cudaMalloc(&sc.base[0], (size_t)k * sizeof(int)));
   TB_CUDA(c, cudaMalloc(&sc.base[1], (size_t)k * sizeof(int)));
   TB_CUDA(c, cudaMalloc(&sc.fit, 1024 * sizeof(double)));
@@ -132,7 +154,7 @@ int tb_knockout(tb_ctx* c, const int32_t* genome, int k, int slot, double h2, in
   int i = 0;
   while (i < k && L >= 2) {
     const int B = std::min(std::min(B_next, 1024), k - i);
-    if (int rc = score_batch(c, sc.base[cur], L, kept_before, B, slot, h2, mode_rule, sc.fit, h)) return rc;
+    if (int rc = score_batch(c, sc, sc.base[cur], L, kept_before, B, slot, h2, mode_rule, sc.fit, h)) return rc;
     ++batches;
     int used = B;
     bool accepted = false;

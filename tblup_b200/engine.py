@@ -114,7 +114,6 @@ class GblupEngine:
             self._ctx = C.c_void_p()
             raise RuntimeError("tb_create failed (%d): %s" % (rc, self._lib.tb_last_error(None).decode()))
         self.device = int(device)
-        self._n_staged = 0
 
     # -- lifetime ------------------------------------------------------------------------------
     def clone(self, device):
@@ -127,7 +126,7 @@ class GblupEngine:
         if rc != 0:
             other._ctx = C.c_void_p()
             raise RuntimeError("tb_clone failed (%d): %s" % (rc, self._lib.tb_last_error(None).decode()))
-        other.n, other.m, other.storage, other.device, other._n_staged = self.n, self.m, self.storage, int(device), 0
+        other.n, other.m, other.storage, other.device = self.n, self.m, self.storage, int(device)
         other.has_phenotypes = self.has_phenotypes
         return other
 
@@ -173,17 +172,24 @@ class GblupEngine:
         off = np.ascontiguousarray(off, dtype=np.int64)
         self._check(self._lib.tb_stage_genomes(self._ctx, flat.ctypes.data, off.ctypes.data, off.size - 1),
                     "tb_stage_genomes")
-        self._n_staged = off.size - 1
 
     def evaluate_staged(self, slots=(0,), h2=0.4, mode=MODE_AUTO, out=None, out_device_ptr=None):
-        """Fitness of the staged batch on each row set -> array (P, n_slots), or written to a device pointer."""
+        """Fitness of the staged batch on each row set -> array (P, n_slots), or written to a device pointer (room for
+        P n_slots doubles).  P is what the library holds staged (``info("staged")``): the batch of the last ``stage`` /
+        ``evaluate``, or the last generation of a ``DeviceDE``, which stages its own batch.  A host ``out`` must be a
+        C-contiguous float64 array of at least P n_slots entries."""
         s = np.ascontiguousarray(np.asarray(slots, dtype=np.int32))
         if out_device_ptr is not None:
             self._check(self._lib.tb_eval_staged(self._ctx, s.ctypes.data, s.size, float(h2), int(mode),
                                                  C.c_void_p(int(out_device_ptr)), 1), "tb_eval_staged")
             return None
+        P = self.info("staged")
         if out is None:
-            out = np.empty((self._n_staged, s.size), dtype=np.float64)
+            out = np.empty((P, s.size), dtype=np.float64)
+        elif not (isinstance(out, np.ndarray) and out.dtype == np.float64 and out.flags.c_contiguous
+                  and out.flags.writeable and out.size >= P * s.size):
+            raise ValueError("evaluate_staged: out must be a writeable C-contiguous float64 array of at least %d x %d "
+                             "entries (%d genomes staged)" % (P, s.size, P))
         self._check(self._lib.tb_eval_staged(self._ctx, s.ctypes.data, s.size, float(h2), int(mode),
                                              out.ctypes.data, 0), "tb_eval_staged")
         return out
@@ -200,7 +206,6 @@ class GblupEngine:
             out = np.empty((P, s.size), dtype=np.float64)
         self._check(self._lib.tb_eval(self._ctx, s.ctypes.data, s.size, flat.ctypes.data, off.ctypes.data, P,
                                       float(h2), int(mode), out.ctypes.data), "tb_eval")
-        self._n_staged = P
         return out
 
     # -- panel models: marker effects and breeding values -----------------------------------------
